@@ -23,14 +23,20 @@ build, fixed stiffness, error against the oracle), `--model softball|softcylinde
             softbox volume mode is linearly unstable, SURVEY App. E: those worlds are flagged diverged and counted).
 `sensor_trace_error`: (N=1) worlds just simulated against the fp64 oracle with the same parameters.
 `traj_kernels`: (N=1, outside the timed region) the HBM-bound kernels that post-process the trajectory buffer.
+`--dump-outputs DIR`: the trajectories of the last timed step (a seeded sample of at most 56 MiB) as DIR/traj.npy; the
+            inputs are a function of the arguments alone, so two builds run with the same arguments compare output for output.
 """
 import argparse
+import atexit
 import ctypes as C
+import functools
 import importlib
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -39,6 +45,8 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+if __name__ == "__main__":
+    sys.dont_write_bytecode = True       # the benchmark leaves the tree as it found it (no __pycache__ of the modules it imports)
 
 STEPS_PER_EPISODE = 1 + 200 * 7
 METRIC = "world-steps/sec"
@@ -161,9 +169,20 @@ def world_params(args, ids, it, mode=None):
 _W = {}
 
 
-def _cpu_init(blob_path, tendon_damping=None):
+@functools.lru_cache(maxsize=None)
+def native_oracle():
+    """Path of the -O3 -march=native oracle, built once per run for the host this runs on.  It goes to a temporary
+    directory, removed at exit, because the tree bench.py runs from may be read-only."""
     from oracle import sgoracle as so
-    so.use_native()                                  # -O3 -march=native, built on the box this runs on
+    d = tempfile.mkdtemp(prefix="softgrip-bench-")
+    atexit.register(shutil.rmtree, d, True)
+    return so.build_native(d)
+
+
+def _cpu_init(blob_path, tendon_damping=None, native=None):
+    """Worker set-up; `native`: the library native_oracle() built in the parent (None: this process builds it)."""
+    from oracle import sgoracle as so
+    so.use_native(native or native_oracle())
     blob = open(blob_path, "rb").read()
     _W["m"] = so.OracleModel(blob)
     _W["w"] = so.OracleWorld(_W["m"])
@@ -222,11 +241,9 @@ def cpu_throughput(args, blob_path, episodes_per_core, repeats=1, cores=None):
     """world-steps/s of the oracle with one process per host core on the bench's own workload; returns
     (value, cores, seconds, sample text, flops per world-step (PGS, all stages))."""
     from concurrent.futures import ProcessPoolExecutor
-    from oracle import sgoracle as so
-    so.build_native(force=True)                      # once, here, for the host this runs on; the workers only load it
     cores = cores or len(os.sched_getaffinity(0))
     best = None
-    with ProcessPoolExecutor(cores, initializer=_cpu_init, initargs=(blob_path, args.tendon_damping)) as ex:
+    with ProcessPoolExecutor(cores, initializer=_cpu_init, initargs=(blob_path, args.tendon_damping, native_oracle())) as ex:
         list(ex.map(_cpu_episodes, [([], None, None)] * cores))      # spin the workers up (model load excluded)
         for rep in range(repeats):
             jobs = _cpu_jobs(args, cores, episodes_per_core, 500000 + rep)
@@ -284,11 +301,10 @@ def run_reference_arm(args, rank):
     blob = os.path.join(ROOT, "tests", "golden", args.model + ".sgm")
     from oracle import sgoracle as so
     so.build()
-    so.build_native(force=True)                      # once, here, for the host this runs on; the workers only load it
     cores = len(os.sched_getaffinity(0))
     from concurrent.futures import ProcessPoolExecutor
     times = []
-    with ProcessPoolExecutor(cores, initializer=_cpu_init, initargs=(blob, args.tendon_damping)) as ex:
+    with ProcessPoolExecutor(cores, initializer=_cpu_init, initargs=(blob, args.tendon_damping, native_oracle())) as ex:
         list(ex.map(_cpu_episodes, [([], None, None)] * cores))
         for it in range(args.warmup + args.steps):
             jobs = _cpu_jobs(args, cores, args.ref_episodes_per_core, it)
@@ -375,6 +391,22 @@ def measure_traj_kernels(torch, traj, flush, hbm_peak, reps=5):
         return {"error": "%s: %s" % (type(e).__name__, e)}
 
 
+DUMP_BYTES = 56 << 20
+
+
+def dump_outputs(out_dir, traj, lo):
+    """--dump-outputs: what the timed rollout returned in its last step, so that two builds can be compared output for output
+    on identical inputs.  traj.npy: the trajectories [n, T, 12] in the batch precision of a fixed, seeded sample of this
+    rank's worlds (all of them when they fit in DUMP_BYTES); traj_worlds.npy: their global world ids (float64)."""
+    import torch
+    W = traj.shape[0]
+    n = min(W, DUMP_BYTES // (traj[0].numel() * traj.element_size()))
+    idx = np.arange(W) if n == W else np.sort(np.random.default_rng(0).choice(W, n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "traj.npy"), traj[torch.as_tensor(idx, device=traj.device)].cpu().numpy())
+    np.save(os.path.join(out_dir, "traj_worlds.npy"), (lo + idx).astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -402,7 +434,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-variants", action="store_true")
     ap.add_argument("--trace-worlds", type=int, default=8)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the trajectories of the last one to DIR/*.npy (rank 0, CUDA path)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed; the reference arm keeps no trajectories")
     if args.warmup < 3:
         args.warmup = 3                      # timing rules: W >= 3
     defaults = {2: ("softbox", 65536, 32, "all", None), 1: ("softbox", 4096, 64, "stiffness", 700.0), 4: ("softbox_refined", 16384, 32, "all", None)}[args.config]
@@ -496,6 +532,8 @@ def main():
     last = args.warmup + args.steps - 1                  # `traj` still holds the last timed step
     pick = sorted(set(int(x) for x in np.linspace(0, Wg - 1, max(1, args.trace_worlds))))
     traj_pick = traj[pick].double().cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, traj, lo)                  # before the variants below reuse `traj`
 
     # ---- end to end through the C-ABI with pinned HOST buffers ----
     k_host = torch.empty(Wg, dtype=torch.float64).pin_memory()

@@ -26,25 +26,23 @@ def build(force=False):
     return so
 
 
-def build_native(force=False):
-    """-O3 -march=native build for the CPU arm of bench.py, compiled on the box it runs on (falls back to the portable
-    build when the compiler is missing); same arithmetic, same results.  The parent process builds it once (force=True)
-    before it starts its workers; the workers only load it."""
-    so = os.path.join(_HERE, "_native", "libsgoracle_native.so")
-    src = os.path.join(_HERE, "sg_oracle.c")
+def build_native(out_dir):
+    """-O3 -march=native build for the CPU arm of bench.py, compiled on the box it runs on into `out_dir` (the source tree
+    may be read-only), falling back to the portable build when the compiler is missing; same arithmetic, same results.
+    Returns the library's path.  The parent process builds it once before it starts its workers; the workers only load it."""
+    so = os.path.join(os.path.abspath(out_dir), "libsgoracle_native.so")
     try:
-        if force or not os.path.exists(so) or os.path.getmtime(so) < os.path.getmtime(src):
-            subprocess.check_call(["make", "-C", _HERE, "-B", "_native/libsgoracle_native.so"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        subprocess.check_call(["make", "-C", _HERE, "-B", "NATIVE=" + so, so], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
         return so
     except Exception:
         return build()
 
 
-def use_native(force=False):
-    """Switch this process to the native build (call before the first lib())."""
-    global _LIB, _NATIVE
+def use_native(path):
+    """Switch this process to the library at `path`, as returned by build_native (call before the first lib())."""
+    global _NATIVE
     if _LIB is None:
-        _NATIVE = build_native(force)
+        _NATIVE = path
 
 
 _NATIVE = None

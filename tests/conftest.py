@@ -9,7 +9,8 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE = os.environ.get("SOFTGRIP_REFERENCE", "/root/reference")
+# a checkout of the upstream soft-grip repository (its data/gripper MJCF files); the tests that read it skip without it
+REFERENCE = os.environ.get("SOFTGRIP_REFERENCE", "")
 
 
 def pytest_configure(config):

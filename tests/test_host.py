@@ -334,6 +334,30 @@ def test_bench_world_params_do_not_depend_on_the_sharding():
     assert np.all(bench.world_params(args, np.arange(8), 0)[0] == 700.0)
 
 
+def test_bench_dump_outputs_is_a_fixed_bounded_sample(tmp_path):
+    """bench.py --dump-outputs: the whole trajectory buffer when it fits, otherwise the same seeded sample of worlds on every
+    run, in the batch precision, under 64 MB in all, with the global ids of the worlds it holds."""
+    torch = pytest.importorskip("torch")
+    sys.path.insert(0, ROOT)
+    import bench
+    small = torch.arange(5 * 200 * 12, dtype=torch.float32).reshape(5, 200, 12)
+    bench.dump_outputs(str(tmp_path / "small"), small, 10)
+    assert np.array_equal(np.load(str(tmp_path / "small" / "traj.npy")), small.numpy())
+    assert np.array_equal(np.load(str(tmp_path / "small" / "traj_worlds.npy")), np.arange(10.0, 15.0))
+    big = torch.randn(4096, 200, 12, dtype=torch.float64, generator=torch.Generator().manual_seed(0))
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), big, 100)
+    files = sorted(os.listdir(str(tmp_path / "a")))
+    assert files == ["traj.npy", "traj_worlds.npy"]
+    assert sum(os.path.getsize(str(tmp_path / "a" / f)) for f in files) <= 64 * 10 ** 6
+    ids = np.load(str(tmp_path / "a" / "traj_worlds.npy"))
+    traj = np.load(str(tmp_path / "a" / "traj.npy"))
+    assert ids.dtype == np.float64 and traj.dtype == np.float64 and 1000 < len(ids) < 4096 and (np.diff(ids) > 0).all()
+    assert np.array_equal(traj, big.numpy()[ids.astype(int) - 100])
+    for f in files:
+        assert np.array_equal(np.load(str(tmp_path / "a" / f)), np.load(str(tmp_path / "b" / f)))
+
+
 def test_regenerate_multi_rank_noise_flags_and_statistics(tmp_path):
     """ADVICE r1: the multi-rank path passes the noise seed to the */train files (a draw depends on the global world id only, so
     the merged file equals the single-rank one), counts every status flag, drops every flagged world, and writes the per-file
