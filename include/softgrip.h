@@ -147,7 +147,7 @@ int sg_batch_debug_get(sg_batch* b, const char* key, double* out, int cap);
 
 /* launch geometry chosen for this batch (host ints, out[8]): [0] lanes per world, [1] warps per CTA, [2] worlds per CTA,
  * [3] resident CTAs per SM, [4] dynamic shared memory per CTA (bytes), [5] shared memory per world (bytes),
- * [6] 0 (was: team mode, removed), [7] kernel generation.
+ * [6] 0 (was: team mode, removed), [7] kernel generation (always 2: sg_step_kernel2).
  * No reference counterpart: it only documents how the worlds were packed onto the SMs (bench.py reports it). */
 int sg_batch_config(const sg_batch* b, int* out);
 

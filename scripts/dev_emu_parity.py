@@ -1,5 +1,5 @@
 """Dev tool: single-step parity of the kernel source (run under the SIMT emulator, no GPU) against the oracle along
-an oracle trajectory.  usage: dev_emu_parity.py [model] [64|32] [nsteps] [lpw] [aux_smem] [stride]"""
+an oracle trajectory.  usage: dev_emu_parity.py [model] [64|32] [nsteps] [lpw] [stride]"""
 import importlib, os, sys, time
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -14,8 +14,7 @@ name = sys.argv[1] if len(sys.argv) > 1 else "softbox"
 prec = int(sys.argv[2]) if len(sys.argv) > 2 else 64
 nsteps = int(sys.argv[3]) if len(sys.argv) > 3 else 400
 lpw = int(sys.argv[4]) if len(sys.argv) > 4 else 8
-aux = int(sys.argv[5]) if len(sys.argv) > 5 else 0
-stride = int(sys.argv[6]) if len(sys.argv) > 6 else 1
+stride = int(sys.argv[5]) if len(sys.argv) > 5 else 1
 blob = os.path.join(ROOT, "tests", "golden", name + ".sgm")
 model = mjcf.load_blob(blob)
 om = so.OracleModel(open(blob, "rb").read())
@@ -24,10 +23,10 @@ ow.set_geom_mask(batched.geom_name_mask(model.names["geom"], "OBJ", ("g12", "g2"
 k = 700.0
 ow.set_stiffness(k)
 W = 32 // lpw + 1
-env = emu.EmuBatch(blob, W, prec=prec, lpw=lpw, aux_smem=aux)
+env = emu.EmuBatch(blob, W, prec=prec, lpw=lpw)
 env.set_params(stiffness=np.full(W, k))
 env.set_debug_world(1)
-print("info nv", env.info.nv, "levels", env.info.nlevels, "maxcon", env.info.maxcon, "smem32", env.info.smem_bytes32, "W", W, "lpw", lpw, "aux_smem", aux)
+print("info nv", env.info.nv, "levels", env.info.nlevels, "maxcon", env.info.maxcon, "smem32", env.info.smem_bytes32, "W", W, "lpw", lpw)
 ow.reset()
 worst = {}
 def rel(a, b):

@@ -1,5 +1,5 @@
 """Dev tool: SM cycles per phase of the step kernel (SOFTGRIP_PROF=1), split into the contact-free settle part and the
-whole episode.  usage: dev_phase.py [model] [W] [configs...]   config = l<lpw>:n<warps>:t<team>:a<aux in shared memory>"""
+whole episode.  usage: dev_phase.py [model] [W] [configs...]   config = l<lpw>:n<warps>"""
 import importlib, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -8,13 +8,11 @@ import torch
 batched = importlib.import_module("soft-grip_b200.batched")
 name = sys.argv[1] if len(sys.argv) > 1 else "softbox"
 W = int(sys.argv[2]) if len(sys.argv) > 2 else 18944
-cfgs = sys.argv[3:] or ["l8:n16:t0"]
+cfgs = sys.argv[3:] or ["l8:n16"]
 dm = batched.DeviceModel(os.path.join(ROOT, "tests", "golden", name + ".sgm"))
 for cfg in cfgs:
     parts = {x[0]: int(x[1:]) for x in cfg.split(":")}
     os.environ["SOFTGRIP_LPW"] = str(parts.get("l", 8))
-    os.environ.pop("SOFTGRIP_TEAM", None)
-    os.environ.pop("SOFTGRIP_AUX_SMEM", None)
     if "n" in parts: os.environ["SOFTGRIP_NW"] = str(parts["n"])
     else: os.environ.pop("SOFTGRIP_NW", None)
     env = batched.BatchedManEnv(dm, W, dtype=torch.float32, seed=0)

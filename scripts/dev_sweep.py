@@ -1,5 +1,5 @@
-"""Dev tool: throughput of the rollout kernel over kernel generation / lanes-per-world / aux placement.
-usage: dev_sweep.py [model] [W] [rows] [configs...]   config = k<kernel>:l<lpw>:a<aux_smem>:n<warps per CTA>"""
+"""Dev tool: throughput of the rollout kernel over lanes-per-world / warps per CTA / the development switches.
+usage: dev_sweep.py [model] [W] [rows] [configs...]   config = l<lpw>:n<warps per CTA>[:<letter><value>...], letters below"""
 import importlib, os, sys, time
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -9,19 +9,19 @@ batched = importlib.import_module("soft-grip_b200.batched")
 name = sys.argv[1] if len(sys.argv) > 1 else "softbox"
 W = int(sys.argv[2]) if len(sys.argv) > 2 else 8192
 rows = int(sys.argv[3]) if len(sys.argv) > 3 else 60
-cfgs = sys.argv[4:] or ["k1:l32:a1", "k2:l8:a0", "k2:l4:a0", "k2:l16:a0", "k2:l32:a0", "k2:l32:a1", "k2:l16:a1"]
+cfgs = sys.argv[4:] or ["l8", "l4", "l16", "l32"]
 blob = os.path.join(ROOT, "tests", "golden", name + ".sgm")
 ev, val = batched.default_schedule(2) if rows == 200 else batched.default_schedule(2, n_settle=10, n_iter=rows - 10, open_close_div=(rows - 10) // 2)
 ref = None
 for cfg in cfgs:
     parts = {x[0]: int(x[1:]) for x in cfg.split(":")}
-    k, l, a = parts.get("k", 2), parts.get("l", 8), parts.get("a", 0)
-    os.environ["SOFTGRIP_LPW"] = str(l); os.environ.pop("SOFTGRIP_AUX_SMEM", None)
-    os.environ.pop("SOFTGRIP_QV_SMEM", None)
-    os.environ.pop("SOFTGRIP_TEAM", None)
+    os.environ["SOFTGRIP_LPW"] = str(parts.get("l", 8))
+    # b0: plain list schedule of the equality sweep instead of the bank-conflict-aware one
     if parts.get("b", 1) == 0: os.environ["SOFTGRIP_NO_BANK_SCHEDULE"] = "1"
     else: os.environ.pop("SOFTGRIP_NO_BANK_SCHEDULE", None)
+    # s0: no CTA barrier at the start of every physics step
     os.environ["SOFTGRIP_STEP_BARRIER"] = str(parts.get("s", 1))
+    # m<n>: contact capacity per world
     if "m" in parts: os.environ["SOFTGRIP_MAXCON"] = str(parts["m"])
     else: os.environ.pop("SOFTGRIP_MAXCON", None)
     # t0 / t1: equality rows in shared memory / forced into tensor memory (default: the library decides)
@@ -30,9 +30,6 @@ for cfg in cfgs:
     # r0: contact records read from the scratch instead of the shared-memory ring
     if "r" in parts: os.environ["SOFTGRIP_RING"] = str(parts["r"])
     else: os.environ.pop("SOFTGRIP_RING", None)
-    # g0: rows_and_smooth gathers the slider state from the scratch instead of its shared-memory copy
-    if "g" in parts: os.environ["SOFTGRIP_STAGE"] = str(parts["g"])
-    else: os.environ.pop("SOFTGRIP_STAGE", None)
     # d0: fixed shares of the world batches per persistent CTA instead of the dynamic hand-out
     if "d" in parts: os.environ["SOFTGRIP_DYNAMIC"] = str(parts["d"])
     else: os.environ.pop("SOFTGRIP_DYNAMIC", None)

@@ -12,8 +12,6 @@
 
 #include "../../include/softgrip.h"
 #include "sg_plan.hpp"
-#define SG_ST_CON_FULL_BIT 2
-#define SG_ST_UNSUPPORTED_BIT 8
 #include "sg_launch.hpp"
 #include "sg_traj.cuh"
 
@@ -33,16 +31,14 @@ struct sg_batch {
   PlanDims D;                 // with per-batch capacities and masks folded in
   int W, device, precision;
   size_t esize;
-  int kernel = 2;             // kernel generation (sg_kernels2.cuh: sub-warp worlds); the first-generation kernel is gone
-  int lpw = 8;                // lanes per world of kernel 2
-  int nwarp = 16;             // warps per CTA of kernel 2
+  int lpw = 8;                // lanes per world
+  int nwarp = 16;             // warps per CTA
   int tm_cols = 0, tm_stride = 0;   // tensor-memory window of the equality rows (KArgs2::tm_cols, tm_stride); 0: shared memory
   int rec_ring = 0;                 // contact records through a shared-memory ring in the freed row region (KArgs2::rec_ring)
-  size_t smem2 = 0;           // dynamic shared memory per CTA of kernel 2
+  size_t smem2 = 0;           // dynamic shared memory per CTA
   Layout2 L2;
-  unsigned char* scratch = nullptr;   // global aux slots of kernel 2 (when aux is not in shared memory)
-  std::vector<int> step_d;            // level-sweep step tables of kernel 2 for this batch's lanes per world
-  std::vector<double> step_iw;
+  unsigned char* scratch = nullptr;   // global aux slots of the worlds (KArgs2::scratch)
+  std::vector<int> step_d;            // level-sweep step tables for this batch's lanes per world
   std::vector<int> row_perm;          // plan schedule position -> storage position of the row in this batch's kernel tables
   void* tab = nullptr;        // device table in batch precision
   int* itab = nullptr;
@@ -56,7 +52,7 @@ struct sg_batch {
   int* stage_touch = nullptr; size_t stage_touch_bytes = 0;
   long long launches = 0;
   int traj_soa = 0;           // trajectory layout of sg_batch_rollout: 0 = [W][T][C], 1 = [T][C][W]
-  unsigned long long* prof = nullptr; size_t prof_n = 0;   // SOFTGRIP_PROF=1: phase clocks of kernel 2 (development aid)
+  unsigned long long* prof = nullptr; size_t prof_n = 0;   // SOFTGRIP_PROF=1: phase clocks of the step kernel (development aid)
   int* batch_counter = nullptr;     // KArgs2::batch_counter (dynamic hand-out of world batches to the persistent CTAs)
   int max_ctas = 0, per_sm = 0;
 };
@@ -93,7 +89,7 @@ extern "C" int sg_model_info(const sg_model* m, sg_info* out) {
   D.maxcon = m->maxcon_default; D.maxcand = m->maxcand_default;
   out->nv = D.nv; out->nfinger = D.nfd; out->nshell = D.ns; out->neq = m->plan.neq; out->nu = D.nu; out->nsensordata = D.nsd;
   out->nlevels = D.nlev; out->maxcon = D.maxcon; out->ngeom = m->plan.ngeom;
-  out->smem_bytes32 = make_layout2<float>(D, 0, 4, 8).smem_stride; out->smem_bytes64 = make_layout2<double>(D, 0, 4, 8).smem_stride;
+  out->smem_bytes32 = make_layout2<float>(D, 4, 8).smem_stride; out->smem_bytes64 = make_layout2<double>(D, 4, 8).smem_stride;
   return 0;
 }
 
@@ -122,29 +118,25 @@ extern "C" int sg_model_set_geom_mask(sg_model* m, const int* mask) {
 static void host_tables(const sg_batch* b, std::vector<double>& tab, std::vector<int>& itab) {
   const Plan& P = b->model->plan;
   tab = P.tab; itab = P.itab;
-  if (b->kernel == 2 && !b->row_perm.empty()) {
-    // kernel 2 stores the equality rows at the positions its step schedule chose (bank-conflict-free steps)
-    const PlanDims& D = P.d;
-    const std::vector<int>& perm = b->row_perm;
-    for (int p = 0; p < D.nrow; p++) {
-      const int q = perm[p];
-      itab[D.io_row_d1 + q] = P.itab[D.io_row_d1 + p]; itab[D.io_row_d2 + q] = P.itab[D.io_row_d2 + p];
-      itab[D.io_row_d12 + q] = P.itab[D.io_row_d12 + p];
-      tab[D.o_row_iw + 2 * q] = P.tab[D.o_row_iw + 2 * p]; tab[D.o_row_iw + 2 * q + 1] = P.tab[D.o_row_iw + 2 * p + 1];
-    }
-    // rows of each slider for the warm start: row position | other slider << 12 (0xfff: none) | "second slider" << 24
-    for (int i = 0; i < D.ns * MAXDOFROWS; i++) {
-      const int code = P.itab[D.io_dof_rows + i];
-      if (code < 0) continue;
-      const int p = code >> 1, second = code & 1;
-      const int d1 = P.itab[D.io_row_d1 + p], d2 = P.itab[D.io_row_d2 + p];
-      const int other = second ? d1 : (d2 >= 0 ? d2 : 0xfff);
-      itab[D.io_dof_rows + i] = perm[p] | (other << 12) | (second << 24);
-    }
+  // the kernel stores the equality rows at the positions its step schedule chose (bank-conflict-free steps)
+  const PlanDims& D = P.d;
+  const std::vector<int>& perm = b->row_perm;
+  for (int p = 0; p < D.nrow; p++) {
+    const int q = perm[p];
+    itab[D.io_row_d1 + q] = P.itab[D.io_row_d1 + p]; itab[D.io_row_d2 + q] = P.itab[D.io_row_d2 + p];
+    itab[D.io_row_d12 + q] = P.itab[D.io_row_d12 + p];
+    tab[D.o_row_iw + 2 * q] = P.tab[D.o_row_iw + 2 * p]; tab[D.o_row_iw + 2 * q + 1] = P.tab[D.o_row_iw + 2 * p + 1];
   }
-  while (tab.size() % 4) tab.push_back(0.0);
+  // rows of each slider for the warm start: row position | other slider << 12 (0xfff: none) | "second slider" << 24
+  for (int i = 0; i < D.ns * MAXDOFROWS; i++) {
+    const int code = P.itab[D.io_dof_rows + i];
+    if (code < 0) continue;
+    const int p = code >> 1, second = code & 1;
+    const int d1 = P.itab[D.io_row_d1 + p], d2 = P.itab[D.io_row_d2 + p];
+    const int other = second ? d1 : (d2 >= 0 ? d2 : 0xfff);
+    itab[D.io_dof_rows + i] = perm[p] | (other << 12) | (second << 24);
+  }
   while (itab.size() % 4) itab.push_back(0);
-  tab.insert(tab.end(), b->step_iw.begin(), b->step_iw.end());
   itab.insert(itab.end(), b->step_d.begin(), b->step_d.end());
 }
 
@@ -210,35 +202,25 @@ static int batch_create_body(const sg_model* m, int nworlds, int device, int pre
   b->D.maxcon = m->maxcon_default; b->D.maxcand = m->maxcand_default;
   cudaDeviceProp prop;
   CUDA_OK(cudaGetDeviceProperties(&prop, device));
-  // kernel selection (environment overrides are development knobs; the defaults are the measured best)
+  // launch configuration (environment overrides are development knobs; the defaults are the measured best)
   // lanes per world: 8 for the committed models (measured best for softbox, softball; within 9 % for softcylinder), 32 for
   // shells beyond 256 elements, where shared memory leaves few worlds per SM and the equality sweep is twice as long at 8
   // lanes (softbox_refined, 434 elements: 1.11e6 / 1.48e6 / 1.72e6 world-steps/s at 8 / 16 / 32 lanes, profiles/r02a_*)
-  b->kernel = 2; b->lpw = b->D.ns > 256 ? 32 : 8; b->nwarp = 16;
-  int aux_in_smem = 0;
+  b->lpw = b->D.ns > 256 ? 32 : 8; b->nwarp = 16;
   if (const char* e = std::getenv("SOFTGRIP_LPW")) b->lpw = std::atoi(e);
   if (const char* e = std::getenv("SOFTGRIP_NW")) b->nwarp = std::atoi(e);
-  int qv_in_smem = 0;
+  int aux_in_smem = 0, qv_in_smem = 0;
   if (const char* e = std::getenv("SOFTGRIP_QV_SMEM")) qv_in_smem = std::atoi(e);
   if (const char* e = std::getenv("SOFTGRIP_AUX_SMEM")) aux_in_smem = std::atoi(e);
-  if (b->kernel == 2 && (aux_in_smem || qv_in_smem)) {
-    return fail("SOFTGRIP_AUX_SMEM / SOFTGRIP_QV_SMEM: the shared-memory placement of the once-per-step data was removed from kernel 2 (measured slower; a single address space lets the compiler emit global loads)");
+  if (aux_in_smem || qv_in_smem) {
+    return fail("SOFTGRIP_AUX_SMEM / SOFTGRIP_QV_SMEM: the shared-memory placement of the once-per-step data was removed from the step kernel (measured slower; a single address space lets the compiler emit global loads)");
   }
   if (b->nwarp < 1 || b->nwarp > SG_MAX_WARPS) { return fail("SOFTGRIP_NW must be 1..16"); }
   if (b->lpw != 4 && b->lpw != 8 && b->lpw != 16 && b->lpw != 32) { return fail("SOFTGRIP_LPW must be 4, 8, 16 or 32"); }
-  if (b->kernel == 2) {
-    const Plan& P = m->plan;
-#if SG_EQ2 && SG_SLOT8
-    build_step_tables2(b->D, P.itab, b->lpw, (int)b->esize, b->step_d, b->row_perm, std::getenv("SOFTGRIP_NO_BANK_SCHEDULE") == nullptr);
-    b->step_iw.clear();
-    b->D.nstep = (int)(b->step_d.size() / (4 * (size_t)b->lpw)) - 1;   // two rows per slot; without the trailing dummy step
-#else
-    build_step_tables(b->D, P.tab, P.itab, b->lpw, (int)b->esize, b->step_d, b->step_iw, b->row_perm, std::getenv("SOFTGRIP_NO_BANK_SCHEDULE") == nullptr);
-    b->D.nstep = (int)(b->step_d.size() / (2 * (size_t)b->lpw)) - 1;   // without the trailing dummy step
-#endif
-    b->D.o_step_iw = (int)((P.tab.size() + 3) / 4 * 4);
-    b->D.io_step_d = (int)((P.itab.size() + 3) / 4 * 4);
-  }
+  const Plan& P = m->plan;
+  build_step_tables(b->D, P.itab, b->lpw, (int)b->esize, b->step_d, b->row_perm, std::getenv("SOFTGRIP_NO_BANK_SCHEDULE") == nullptr);
+  b->D.nstep = (int)(b->step_d.size() / (2 * (size_t)b->lpw)) - 1;   // without the trailing dummy step
+  b->D.io_step_d = (int)((P.itab.size() + 3) / 4 * 4);
   int rc = upload_tables(b, true);
   if (rc) { return rc; }
   const size_t nv = b->D.nv, nu = b->D.nu > 0 ? b->D.nu : 1;
@@ -255,96 +237,87 @@ static int batch_create_body(const sg_model* m, int nworlds, int device, int pre
   b->debug_cap = 64 + 16 * 2 * b->D.maxcon + b->D.nv + 3 * (b->D.nrow + 1 + MAXFD + 3 * b->D.maxcon) + 64 + 2 * (b->D.nrow + 1);
   CUDA_OK(cudaMalloc((void**)&b->debug_out, sizeof(double) * b->debug_cap));
   CUDA_OK(cudaMemset(b->debug_out, 0, sizeof(double) * b->debug_cap));
-  int per_sm = 0;
-  if (b->kernel == 2) {
-    const int wpw = 32 / b->lpw;
-    // Launch geometry.  Warps never exchange data, and the kernel is bound by the dependent-issue latency of each warp
-    // (profiles/r02c_phase_scan.txt: 1.05e6 cycles per warp-step with one warp per SM, 1.58e6 with sixteen), so what
-    // counts is (i) every SM busy and (ii) as few passes over the batch list as possible.  Among the CTA sizes that fit,
-    // take the one with the smallest modelled time  passes * (1 + 0.035 (resident warps - 1));  several small CTAs per SM
-    // are penalised: their warps do not share the per-step barrier, which costs instruction-cache locality
-    // (profiles/r01s_*).  E.g. 8 192 worlds (BASELINE configs[2] on 8 GPUs) run as 147 CTAs of 56 worlds instead of
-    // 128 CTAs of 64 on 148 SMs.
-    const bool nw_forced = std::getenv("SOFTGRIP_NW") != nullptr;
-    int best_nw = 0; double best_cost = 0;
-    for (int nw = nw_forced ? b->nwarp : SG_MAX_WARPS; nw >= (nw_forced ? b->nwarp : 1); nw--) {
-      const Layout2 L = precision == 32 ? make_layout2<float>(b->D, aux_in_smem, wpw, b->lpw, qv_in_smem) : make_layout2<double>(b->D, aux_in_smem, wpw, b->lpw, qv_in_smem);
-      const size_t smem = (size_t)L.smem_tables + (size_t)L.smem_stride * wpw * nw;
-      if (smem > prop.sharedMemPerBlockOptin) continue;
-      int ps = 0;
-      const int e = k2_dispatch_configure(precision, b->lpw, 32 * nw, smem, &ps);
-      if (e == -12345) { return fail("SOFTGRIP_LPW: this lanes-per-world value is not compiled in"); }
-      if (e) { return fail(std::string("kernel configuration failed: ") + cudaGetErrorString((cudaError_t)e)); }
-      if (ps < 1) continue;
-      const long ctas = ((long)nworlds + nw * wpw - 1) / (nw * wpw);
-      const long resident = (long)ps * prop.multiProcessorCount;
-      const long passes = (ctas + resident - 1) / resident;
-      const long per_sm_used = ctas < resident ? (ctas + prop.multiProcessorCount - 1) / prop.multiProcessorCount : ps;
-      double cost = (double)passes * (1.0 + 0.035 * (double)(per_sm_used * nw - 1));
-      if (per_sm_used > 1) cost *= 1.3;
-      if (!best_nw || cost < best_cost * (1.0 - 1e-9)) { best_nw = nw; best_cost = cost; }
-    }
-    if (!best_nw) { return fail("sg_batch_create: worlds of one warp do not fit in shared memory (use more lanes per world)"); }
-    b->nwarp = best_nw;
-    b->L2 = precision == 32 ? make_layout2<float>(b->D, aux_in_smem, wpw, b->lpw, qv_in_smem) : make_layout2<double>(b->D, aux_in_smem, wpw, b->lpw, qv_in_smem);
-    b->smem2 = (size_t)b->L2.smem_tables + (size_t)b->L2.smem_stride * wpw * b->nwarp;
-#if SG_SLOT8
-    {
-      // the 8-byte step slots and the unit-coefficient tendon row assume what every MuJoCo composite has: one element mass
-      // and coefficient 1 for every slider of the volume tendon
-      const Plan& P = m->plan;
-      bool uniform = true;
-      for (int e = 0; e < b->D.ns; e++)
-        if (P.tab[b->D.o_sl_m + e] != P.tab[b->D.o_sl_m] || P.tab[b->D.o_sl_tc + e] != 1.0) uniform = false;
-      if (!uniform) { return fail("sg_batch_create: shell elements with different masses or tendon coefficients are not supported by this build (SG_SLOT8)"); }
-    }
-#endif
-    if (b->D.nrow >= 0xfff || b->D.ns >= 0xfff) { return fail("sg_batch_create: too many equality rows or shell joints for the packed warm-start table"); }
-    if (b->L2.cand_cap < 16) { return fail("sg_batch_create: the collision scratch (the equality-row pairs of one world) is too small for this model"); }
-    if (const char* e = std::getenv("SOFTGRIP_TEAM")) { if (std::atoi(e) != 0) { return fail("SOFTGRIP_TEAM: team mode was removed from kernel 2 (measured slower, profiles/r01b_*, r01g_*)"); } }
-    if (b->smem2 > prop.sharedMemPerBlockOptin) { return fail("sg_batch_create: worlds of one warp do not fit in shared memory (use more lanes per world or SOFTGRIP_AUX_SMEM=0)"); }
-    int e = k2_dispatch_configure(precision, b->lpw, 32 * b->nwarp, b->smem2, &per_sm);
+  const int wpw = 32 / b->lpw;
+  // Launch geometry.  Warps never exchange data, and the kernel is bound by the dependent-issue latency of each warp
+  // (profiles/r02c_phase_scan.txt: 1.05e6 cycles per warp-step with one warp per SM, 1.58e6 with sixteen), so what
+  // counts is (i) every SM busy and (ii) as few passes over the batch list as possible.  Among the CTA sizes that fit,
+  // take the one with the smallest modelled time  passes * (1 + 0.035 (resident warps - 1));  several small CTAs per SM
+  // are penalised: their warps do not share the per-step barrier, which costs instruction-cache locality
+  // (profiles/r01s_*).  E.g. 8 192 worlds (BASELINE configs[2] on 8 GPUs) run as 147 CTAs of 56 worlds instead of
+  // 128 CTAs of 64 on 148 SMs.
+  const bool nw_forced = std::getenv("SOFTGRIP_NW") != nullptr;
+  int best_nw = 0; double best_cost = 0;
+  for (int nw = nw_forced ? b->nwarp : SG_MAX_WARPS; nw >= (nw_forced ? b->nwarp : 1); nw--) {
+    const Layout2 L = precision == 32 ? make_layout2<float>(b->D, wpw, b->lpw) : make_layout2<double>(b->D, wpw, b->lpw);
+    const size_t smem = (size_t)L.smem_tables + (size_t)L.smem_stride * wpw * nw;
+    if (smem > prop.sharedMemPerBlockOptin) continue;
+    int ps = 0;
+    const int e = k2_dispatch_configure(precision, b->lpw, 32 * nw, smem, &ps);
     if (e == -12345) { return fail("SOFTGRIP_LPW: this lanes-per-world value is not compiled in"); }
     if (e) { return fail(std::string("kernel configuration failed: ") + cudaGetErrorString((cudaError_t)e)); }
-    if (per_sm < 1) per_sm = 1;
-    b->max_ctas = per_sm * prop.multiProcessorCount; b->per_sm = per_sm;
-#if !(SG_EQ2 && SG_SLOT8)
-    {
-      // The (u, n) pairs of the equality sweep go to tensor memory when every resident CTA of an SM gets its window:
-      // 2 (fp32) or 4 (fp64) columns per step and one empty step past the end for each warp, four warps (one per lane
-      // quarter) share a column block, 512 columns per SM.  SOFTGRIP_TMEM=0 keeps them in shared memory, =1 takes
-      // tensor memory whenever one CTA fits (further CTAs of the SM then wait for the allocation).
-      const int stride = (b->D.nstep + 1) * (precision == 32 ? 2 : 4);
-      int need = 32;
-      while (need < ((b->nwarp + 3) / 4) * stride) need *= 2;
-      int mode = -1;
-      if (const char* te = std::getenv("SOFTGRIP_TMEM")) mode = std::atoi(te);
-      if (need <= 512 && mode != 0 && (mode == 1 || need * per_sm <= 512)) { b->tm_cols = need; b->tm_stride = stride; }
-      // With the rows in tensor memory their shared-memory region is free during the solve: a two-entry ring of contact
-      // records per lane goes there if it fits (SOFTGRIP_RING=0: records are read from the scratch as before).
-      const size_t esz = precision == 32 ? 4 : 8;
-      const size_t ring_bytes = (size_t)b->lpw * (2 * CR_STRIDE * esz + 16);
-      int ring_mode = 1;
-      if (const char* re = std::getenv("SOFTGRIP_RING")) ring_mode = std::atoi(re);
-      if (b->tm_cols && ring_mode != 0 && ring_bytes <= 2 * (size_t)b->D.nrow * esz) b->rec_ring = 1;
-    }
-#endif
-    const int cta_worlds = wpw * b->nwarp;
-    int need = (nworlds + cta_worlds - 1) / cta_worlds;
-    int slots = need < b->max_ctas ? need : b->max_ctas;
-    if (const char* pe = std::getenv("SOFTGRIP_PROF")) {
-      if (std::atoi(pe) != 0) {
-        b->prof_n = PH_COUNT + (size_t)b->max_ctas * b->nwarp;
-        CUDA_OK(cudaMalloc((void**)&b->prof, sizeof(unsigned long long) * b->prof_n));
-        CUDA_OK(cudaMemset(b->prof, 0, sizeof(unsigned long long) * b->prof_n));
-      }
-    }
-    CUDA_OK(cudaMalloc((void**)&b->batch_counter, sizeof(int)));
-    if (!aux_in_smem) {
-      CUDA_OK(cudaMalloc((void**)&b->scratch, (size_t)slots * cta_worlds * (size_t)b->L2.gs_stride));
-      CUDA_OK(cudaMemset(b->scratch, 0, (size_t)slots * cta_worlds * (size_t)b->L2.gs_stride));
+    if (ps < 1) continue;
+    const long ctas = ((long)nworlds + nw * wpw - 1) / (nw * wpw);
+    const long resident = (long)ps * prop.multiProcessorCount;
+    const long passes = (ctas + resident - 1) / resident;
+    const long per_sm_used = ctas < resident ? (ctas + prop.multiProcessorCount - 1) / prop.multiProcessorCount : ps;
+    double cost = (double)passes * (1.0 + 0.035 * (double)(per_sm_used * nw - 1));
+    if (per_sm_used > 1) cost *= 1.3;
+    if (!best_nw || cost < best_cost * (1.0 - 1e-9)) { best_nw = nw; best_cost = cost; }
+  }
+  if (!best_nw) { return fail("sg_batch_create: worlds of one warp do not fit in shared memory (use more lanes per world)"); }
+  b->nwarp = best_nw;
+  b->L2 = precision == 32 ? make_layout2<float>(b->D, wpw, b->lpw) : make_layout2<double>(b->D, wpw, b->lpw);
+  b->smem2 = (size_t)b->L2.smem_tables + (size_t)b->L2.smem_stride * wpw * b->nwarp;
+  {
+    // the 8-byte step slots and the unit-coefficient tendon row assume what every MuJoCo composite has: one element mass
+    // and coefficient 1 for every slider of the volume tendon
+    bool uniform = true;
+    for (int e = 0; e < b->D.ns; e++)
+      if (P.tab[b->D.o_sl_m + e] != P.tab[b->D.o_sl_m] || P.tab[b->D.o_sl_tc + e] != 1.0) uniform = false;
+    if (!uniform) { return fail("sg_batch_create: shell elements with different masses or tendon coefficients are not supported"); }
+  }
+  if (b->D.nrow >= 0xfff || b->D.ns >= 0xfff) { return fail("sg_batch_create: too many equality rows or shell joints for the packed warm-start table"); }
+  if (b->L2.cand_cap < 16) { return fail("sg_batch_create: the collision scratch (the equality-row pairs of one world) is too small for this model"); }
+  if (const char* e = std::getenv("SOFTGRIP_TEAM")) { if (std::atoi(e) != 0) { return fail("SOFTGRIP_TEAM: team mode was removed from the step kernel (measured slower, profiles/r01b_*, r01g_*)"); } }
+  if (b->smem2 > prop.sharedMemPerBlockOptin) { return fail("sg_batch_create: worlds of one warp do not fit in shared memory (use more lanes per world)"); }
+  int per_sm = 0;
+  const int cfg = k2_dispatch_configure(precision, b->lpw, 32 * b->nwarp, b->smem2, &per_sm);
+  if (cfg == -12345) { return fail("SOFTGRIP_LPW: this lanes-per-world value is not compiled in"); }
+  if (cfg) { return fail(std::string("kernel configuration failed: ") + cudaGetErrorString((cudaError_t)cfg)); }
+  if (per_sm < 1) per_sm = 1;
+  b->max_ctas = per_sm * prop.multiProcessorCount; b->per_sm = per_sm;
+  {
+    // The (u, n) pairs of the equality sweep go to tensor memory when every resident CTA of an SM gets its window:
+    // 2 (fp32) or 4 (fp64) columns per step and one empty step past the end for each warp, four warps (one per lane
+    // quarter) share a column block, 512 columns per SM.  SOFTGRIP_TMEM=0 keeps them in shared memory, =1 takes
+    // tensor memory whenever one CTA fits (further CTAs of the SM then wait for the allocation).
+    const int stride = (b->D.nstep + 1) * (precision == 32 ? 2 : 4);
+    int need = 32;
+    while (need < ((b->nwarp + 3) / 4) * stride) need *= 2;
+    int mode = -1;
+    if (const char* te = std::getenv("SOFTGRIP_TMEM")) mode = std::atoi(te);
+    if (need <= 512 && mode != 0 && (mode == 1 || need * per_sm <= 512)) { b->tm_cols = need; b->tm_stride = stride; }
+    // With the rows in tensor memory their shared-memory region is free during the solve: a two-entry ring of contact
+    // records per lane goes there if it fits (SOFTGRIP_RING=0: records are read from the scratch as before).
+    const size_t esz = precision == 32 ? 4 : 8;
+    const size_t ring_bytes = (size_t)b->lpw * (2 * CR_STRIDE * esz + 16);
+    int ring_mode = 1;
+    if (const char* re = std::getenv("SOFTGRIP_RING")) ring_mode = std::atoi(re);
+    if (b->tm_cols && ring_mode != 0 && ring_bytes <= 2 * (size_t)b->D.nrow * esz) b->rec_ring = 1;
+  }
+  const int cta_worlds = wpw * b->nwarp;
+  int need = (nworlds + cta_worlds - 1) / cta_worlds;
+  int slots = need < b->max_ctas ? need : b->max_ctas;
+  if (const char* pe = std::getenv("SOFTGRIP_PROF")) {
+    if (std::atoi(pe) != 0) {
+      b->prof_n = PH_COUNT + (size_t)b->max_ctas * b->nwarp;
+      CUDA_OK(cudaMalloc((void**)&b->prof, sizeof(unsigned long long) * b->prof_n));
+      CUDA_OK(cudaMemset(b->prof, 0, sizeof(unsigned long long) * b->prof_n));
     }
   }
+  CUDA_OK(cudaMalloc((void**)&b->batch_counter, sizeof(int)));
+  CUDA_OK(cudaMalloc((void**)&b->scratch, (size_t)slots * cta_worlds * (size_t)b->L2.gs_stride));
+  CUDA_OK(cudaMemset(b->scratch, 0, (size_t)slots * cta_worlds * (size_t)b->L2.gs_stride));
   return sg_batch_reset(b, nullptr);
 }
 
@@ -363,9 +336,9 @@ extern "C" long long sg_batch_launch_count(const sg_batch* b) { return b ? b->la
 extern "C" int sg_batch_config(const sg_batch* b, int* out) {
   if (!b || !out) return fail("sg_batch_config: null argument");
   const int wpw = 32 / b->lpw;
-  out[0] = b->kernel == 2 ? b->lpw : 32; out[1] = b->kernel == 2 ? b->nwarp : 1; out[2] = b->kernel == 2 ? wpw * b->nwarp : 1;
-  out[3] = b->per_sm; out[4] = b->kernel == 2 ? (int)b->smem2 : 0; out[5] = b->kernel == 2 ? b->L2.smem_stride : 0;
-  out[6] = 0; out[7] = b->kernel;
+  out[0] = b->lpw; out[1] = b->nwarp; out[2] = wpw * b->nwarp;
+  out[3] = b->per_sm; out[4] = (int)b->smem2; out[5] = b->L2.smem_stride;
+  out[6] = 0; out[7] = 2;
   return 0;
 }
 
@@ -684,15 +657,9 @@ extern "C" int sg_batch_debug_get(sg_batch* b, const char* key, double* out, int
     // host-side tables of the equality sweep (no device data): [nstep, lanes per world, bytes per real, nrow, estimated
     // shared-memory wavefronts per sweep], the slot descriptors (2 ints per slot, nstep + 1 steps), then the storage
     // position of every row (plan schedule order)
-    // (rows per slot: 2 when the sweep takes two rows per lane and step, SG_EQ2 -- then 4 ints per slot; it rides in the
-    // upper digits of the wavefront figure so that the header keeps its five entries)
-#if SG_EQ2 && SG_SLOT8
-    const int rows_per_slot = 2;
-    const long wf = sweep_wavefronts2(b->step_d, b->lpw, (int)b->esize);
-#else
+    // (the rows per slot, always 1, ride in the upper digits of the wavefront figure: 1e9 * rows per slot + wavefronts)
     const int rows_per_slot = 1;
     const long wf = sweep_wavefronts(b->step_d, b->lpw, (int)b->esize);
-#endif
     std::vector<double> t = {(double)b->D.nstep, (double)b->lpw, (double)b->esize, (double)b->D.nrow, (double)wf + 1e9 * rows_per_slot};
     for (int v : b->step_d) t.push_back((double)(unsigned)v);
     for (int v : b->row_perm) t.push_back((double)v);

@@ -34,28 +34,11 @@
 #pragma once
 #include <stdint.h>
 
+#include "../../include/softgrip.h"
 #include "sg_plan.hpp"
 #include "sg_math.cuh"
 
 namespace sg {
-
-
-// how many blocks ahead a chain lane prefetches its contact records into L1 when the shared-memory record ring is not in
-// use.  The L1 left beside 228 KB of shared memory is 28 KB; 16 warps x 8 lanes x 128 B are 16 KB of records in flight
-// per block of look-ahead -- which is why the prefetch does not hold and the ring exists (see chain_phase).
-#ifndef SG_PF_DIST
-#define SG_PF_DIST 2      // 1 and 2 measure the same (profiles/r02o_sweep.log: 1.216e7 / 1.223e7)
-#endif
-
-// 8-byte step slots / unit tendon coefficients for shells with uniform element mass (checked by the host, sg_api.cu)
-#ifndef SG_SLOT8
-#define SG_SLOT8 1
-#endif
-
-#ifndef SG_ST_CON_FULL_BIT
-#define SG_ST_CON_FULL_BIT 2
-#define SG_ST_UNSUPPORTED_BIT 8
-#endif
 
 // contact record: 32 words of T, 16-byte aligned groups
 // Words 15, 26, 27 carry the tangential 2x2 block the way the friction solve wants it -- scaled by the friction coefficient and
@@ -76,9 +59,9 @@ struct Layout2 {
   int hotT;
   int h_misc;            // 8 ints
   int hotI;
-  // aux: shared memory or global scratch
+  // aux: global scratch
   int q, v, qs, jtf, a0; // nv each (qs: qacc_smooth; a0: qacc_warmstart at step entry, for the re-run after a divergence reset)
-  int qv_in_smem, hq, hv; // optionally qpos/qvel live in the hot region (offsets hq, hv) instead of aux
+  int qv_in_smem, hq, hv; // unused, 0 (qpos / qvel in the hot region: a removed variant)
   int act, ctrl, actdot; // nu each
   int s_jv, s_ab, s_rot; // per sensor: 12, 3, 9
   int sens;              // nsd
@@ -90,7 +73,7 @@ struct Layout2 {
   int i_cand;            // (unused since the schedule's time slots moved to the shared-memory scratch)
   int i_lmask;           // MAXCHAIN : active-limit masks (bit jl: lower, bit 4+jl: upper)
   int auxI;
-  int aux_in_smem;
+  int aux_in_smem;       // unused, 0 (aux in shared memory: a removed variant)
   // collision scratch: the (u, n) pairs of the equality rows are dead between the end of the solve and the next
   // rows_and_smooth(), so gripper() and collide() keep their per-step data there (offsets in T words from row2)
   int sc_cen;            // 3*ns : capsule centres
@@ -100,14 +83,14 @@ struct Layout2 {
   int cand_cap;          // capacity of the candidate list (<= 0: the model does not fit the scratch)
   int smem_stride;       // bytes per world in shared memory (multiple of 16, bank-skewed)
   int smem_tables;       // bytes of the CTA-shared level-sweep step tables at the start of shared memory
-  int gs_stride;         // bytes per world in the global scratch (0 when aux_in_smem)
+  int gs_stride;         // bytes per world in the global scratch
 };
 
 enum { M2_NCON = 0, M2_STATUS = 1, M2_TOUCH = 2, M2_NCONTOT = 3, M2_ITERS = 4, M2_NCAND = 5, M2_TMAX = 6, M2_NLIM = 7, M2_DONE = 8,
        M2_LMASK = 9 /* MAXCHAIN entries */ };
 
 template <typename T>
-inline Layout2 make_layout2(const PlanDims& D, int aux_in_smem, int wpw, int lpw, int qv_in_smem = 0) {
+inline Layout2 make_layout2(const PlanDims& D, int wpw, int lpw) {
   Layout2 L{};
   int o = 0;
   auto take = [&](int n) { int r = o; o += (n + 3) & ~3; return r; };   // keep every array 16-byte aligned (float4 loads)
@@ -117,8 +100,6 @@ inline Layout2 make_layout2(const PlanDims& D, int aux_in_smem, int wpw, int lpw
   o = (o + 3) & ~3;
   L.minv = take(16 * MAXCHAIN);          // 4-vector loads
   L.a = pack(D.nv + 1); L.hlim = pack(4 * MAXFD); L.h_impr = pack(1);
-  L.qv_in_smem = qv_in_smem;
-  if (qv_in_smem) { L.hq = pack(D.nv); L.hv = pack(D.nv); }
   o = (o + 1) & ~1;                      // the int block (and a double-precision aux block) stays 8-byte aligned
   L.hotT = o;
   L.h_misc = 0; L.hotI = 12;
@@ -135,15 +116,13 @@ inline Layout2 make_layout2(const PlanDims& D, int aux_in_smem, int wpw, int lpw
   L.i_con = takei(D.maxcon); L.i_tl = takei(D.maxcon); L.i_order = takei(D.maxcon);
   L.i_cand = takei(D.ns); L.i_lmask = takei(MAXCHAIN);
   L.auxI = io;
-  L.aux_in_smem = aux_in_smem;
   size_t hot = sizeof(T) * (size_t)L.hotT + sizeof(int) * (size_t)L.hotI;
   size_t aux = sizeof(T) * (size_t)L.auxT + sizeof(int) * (size_t)L.auxI;
-  size_t sb = hot + (aux_in_smem ? aux : 0);
-  sb = (sb + 15) & ~(size_t)15;
+  size_t sb = (hot + 15) & ~(size_t)15;
   // skew consecutive worlds of a warp by 32/wpw banks so that the same offset in different groups hits different banks
   if (wpw > 1) { const size_t unit = (size_t)(128 / wpw) < 16 ? 16 : (size_t)(128 / wpw); while ((sb / unit) % 2 == 0 || sb % unit) sb += 16; }
   L.smem_stride = (int)sb;
-  L.gs_stride = aux_in_smem ? 0 : (int)((aux + 127) & ~(size_t)127);
+  L.gs_stride = (int)((aux + 127) & ~(size_t)127);
   {
     int so = 0;
     L.sc_cen = so; so += 3 * D.ns > D.ns + 32 ? 3 * D.ns : D.ns + 32;   // later reused for the contact schedule's time slots
@@ -154,9 +133,9 @@ inline Layout2 make_layout2(const PlanDims& D, int aux_in_smem, int wpw, int lpw
     L.cand_cap = (2 * D.nrow - so) * (int)(sizeof(T) / sizeof(int));
     if (L.cand_cap > D.maxcand) L.cand_cap = D.maxcand;
   }
-  // CTA-shared tables: step slots | tendon coefficients, coefficient / mass, 1 / mass (ns each) | slider axes (3 ns) |
-  // collider table | broadphase runs | row -> sliders
-  L.smem_tables = (int)(((size_t)(D.nstep + 1) * lpw * ((SG_EQ2 && SG_SLOT8) ? 16 : SG_SLOT8 ? 8 : 8 + 2 * sizeof(T)) + (6 * (size_t)D.ns + (size_t)MAXCOLL * CO_STRIDE) * sizeof(T) +
+  // CTA-shared tables: step slots (8 bytes) | tendon coefficients, coefficient / mass, 1 / mass (ns each) | slider axes
+  // (3 ns) | collider table | broadphase runs | row -> sliders
+  L.smem_tables = (int)(((size_t)(D.nstep + 1) * lpw * 8 + (6 * (size_t)D.ns + (size_t)MAXCOLL * CO_STRIDE) * sizeof(T) +
                          (4 * (size_t)D.nrun + (size_t)D.nrow) * sizeof(int) + 127) & ~(size_t)127);
   return L;
 }
@@ -207,7 +186,7 @@ struct KArgs2 {
   int tm_cols;                 // tensor-memory columns the CTA allocates (power of two >= 32), 0: the (u, n) rows stay in shared memory
   int tm_stride;               // columns per warp: warp w owns [tm_stride (w / 4), +tm_stride) of its lane quarter
   int rec_ring;                // 1: contact records reach the chain phase through a two-entry shared-memory ring per lane (needs tm_cols)
-  unsigned char* scratch;      // global aux slots [gridDim.x * WPW][L.gs_stride] (null when aux_in_smem)
+  unsigned char* scratch;      // global aux slots [gridDim.x * WPW][L.gs_stride]
   int* batch_counter;          // persistent CTAs take their batches of worlds from this counter (zeroed before the launch);
                                // null: batch i of CTA c is i * gridDim.x + c
   // state, world-major
@@ -244,36 +223,28 @@ template <> __device__ __forceinline__ float trcp<float>(float x) {
 
 // Pins a loop-invariant pointer / value in registers: without it ptxas rebuilds such values from the kernel-parameter
 // bank inside the contact loop (three constant loads plus 64-bit address arithmetic per record pointer, per block).
-#ifndef SG_HOIST
-#define SG_HOIST 1
-#endif
-// the chain's M^-1 block is requested from shared memory before the cost test of a contact block instead of after it:
-// 1.447e7 -> 1.474e7 world-steps/s (profiles/r02zc_sweep.log)
-#ifndef SG_MV_EARLY
-#define SG_MV_EARLY 1
-#endif
 // (the OFFSET is pinned, not the pointer: a pointer that went through an asm statement loses its address space and every
 // access through it becomes a generic load)
 __device__ __forceinline__ long long keep_off(long long o) {
-#if defined(__CUDA_ARCH__) && SG_HOIST
+#if defined(__CUDA_ARCH__)
   asm volatile("" : "+l"(o));
 #endif
   return o;
 }
 __device__ __forceinline__ int keep_off(int o) {
-#if defined(__CUDA_ARCH__) && SG_HOIST
+#if defined(__CUDA_ARCH__)
   asm volatile("" : "+r"(o));
 #endif
   return o;
 }
 __device__ __forceinline__ float keep_val(float x) {
-#if defined(__CUDA_ARCH__) && SG_HOIST
+#if defined(__CUDA_ARCH__)
   asm volatile("" : "+f"(x));
 #endif
   return x;
 }
 __device__ __forceinline__ double keep_val(double x) {
-#if defined(__CUDA_ARCH__) && SG_HOIST
+#if defined(__CUDA_ARCH__)
   asm volatile("" : "+d"(x));
 #endif
   return x;
@@ -474,9 +445,6 @@ __device__ __forceinline__ void friction_fast(float& f1, float& f2, float& la_io
   if (kb == 0.0f) { f1 = 0; f2 = 0; la_io = 0; return; }                  // mju_QCQP2: singular -> zero, inactive
   const float a22 = 1.0f - a11, b1 = bc0 * kb, b2 = bc1 * kb;
   const float rr = trcp<float>(f0);
-#ifndef SG_X_FRIC_MAXIT
-#define SG_X_FRIC_MAXIT 8          // (timing experiments only: a lower cap changes the results)
-#endif
   float lo = tfsqrt<float>(b1 * b1 + b2 * b2) * rr - 1.0f;               // lower bound |b|/r - trace of the root
   if (!(lo > 0.0f)) lo = 0.0f;
   // start from the root of the previous sweep (la_io, in the same normalised units; 0 on the first sweep) when it lies
@@ -485,7 +453,7 @@ __device__ __forceinline__ void friction_fast(float& f1, float& f2, float& la_io
   float la = fmaxf(lo, la_io);
   float w1 = 0, w2 = 0, rdet = 0, N2 = 0;
 #pragma unroll 1
-  for (int iter = 0; iter < SG_X_FRIC_MAXIT; iter++) {
+  for (int iter = 0; iter < 8; iter++) {                                  // a lower cap changes the results
 #if defined(SG_FRIC_STATS) && !defined(__CUDA_ARCH__)
     sg_fric_evals++;
 #endif
@@ -552,19 +520,10 @@ template <> __device__ __forceinline__ void ldg2<float>(const float* p, float& x
 template <> __device__ __forceinline__ void ldg2<double>(const double* p, double& x, double& y) { const double2 v = __ldg(reinterpret_cast<const double2*>(p)); x = v.x; y = v.y; }
 static_assert(MAXCD == 4, "finger chain blocks are loaded as 4-vectors");
 
-// one slot of the level-sweep step tables in shared memory (host encoding: sg_plan.hpp build_step_tables)
-#if SG_EQ2 && SG_SLOT8
-// two rows per lane and step (sg_plan.hpp build_step_tables2): {xA, yA, xB, yB}, one 128-bit shared-memory load
-template <typename T> struct alignas(16) Slot { unsigned x, y, xb, yb; };
-#elif SG_SLOT8
-// uniform shell (every slider has the same mass and tendon coefficient 1, as every MuJoCo composite has): the slot is the
-// 8-byte descriptor alone -- one 64-bit shared-memory load, two wavefronts per warp instead of four
+// one slot of the level-sweep step tables in shared memory (host encoding: sg_plan.hpp build_step_tables).  The shell is
+// uniform (every slider has the same mass and tendon coefficient 1, as every MuJoCo composite has; checked by the host,
+// sg_api.cu), so the slot is the 8-byte descriptor alone -- one 64-bit shared-memory load, two wavefronts per warp
 template <typename T> struct alignas(8) Slot { unsigned x, y; };
-#else
-template <typename T> struct Slot;
-template <> struct alignas(16) Slot<float> { unsigned x, y; float iw1, iw2; };      // one 128-bit shared-memory load
-template <> struct alignas(8) Slot<double> { unsigned x, y; double iw1, iw2; };
-#endif
 template <typename T> __device__ __forceinline__ Slot<T> ld_slot(const Slot<T>* p) { return *p; }
 
 // Once-per-step loops over the sliders / rows of a lane: ptxas does not move the global loads of iteration i + 1 above
@@ -1173,7 +1132,7 @@ struct World2 {
           const unsigned m = gballot(pass);
           if (pass) {
             const int slot = ncand + __popc(m & ((1u << sl) - 1));
-            if (slot < cand_cap) cand[slot] = pt | (pa << 3) | (pb << 8); else flags |= SG_ST_CON_FULL_BIT;
+            if (slot < cand_cap) cand[slot] = pt | (pa << 3) | (pb << 8); else flags |= SG_ST_CON_FULL;
           }
           ncand += __popc(m);
         }
@@ -1209,7 +1168,7 @@ struct World2 {
         const unsigned m = gballot(pass);
         if (pass) {
           const int slot = ncand + __popc(m & ((1u << sl) - 1));
-          if (slot < cand_cap) cand[slot] = pt | (pa << 3) | (pb << 8); else flags |= SG_ST_CON_FULL_BIT;
+          if (slot < cand_cap) cand[slot] = pt | (pa << 3) | (pb << 8); else flags |= SG_ST_CON_FULL;
         }
         ncand += __popc(m);
       }
@@ -1248,8 +1207,8 @@ struct World2 {
           const T* co2 = scoll + pb * CO_STRIDE;
           T c2[3], rot2[9]; collider_pose(pb, c2, rot2);
           T size2[3] = {co2[CO_SIZE], co2[CO_SIZE + 1], co2[CO_SIZE + 2]};
-          if (box_box_overlap(c1, rot1, size1, c2, rot2, size2)) flags |= SG_ST_UNSUPPORTED_BIT;
-        } else flags |= SG_ST_UNSUPPORTED_BIT;
+          if (box_box_overlap(c1, rot1, size1, c2, rot2, size2)) flags |= SG_ST_UNSUPPORTED;
+        } else flags |= SG_ST_UNSUPPORTED;
         if (n > 0) { touch |= (1 << 30); if (mask & 1) touch |= (mask >> 1); }
       }
       // contacts with dist >= 0 (== includemargin) exist but carry no constraint rows
@@ -1262,7 +1221,7 @@ struct World2 {
       for (int i = 0; i < n; i++) {
         if (rc[i].dist < T(0)) {
           if (slot < D.maxcon) contact_rows(slot, rc[i], pa, e, ssign, dbg, dslot + i);
-          else flags |= SG_ST_CON_FULL_BIT;
+          else flags |= SG_ST_CON_FULL;
           slot++;
         }
       }
@@ -1569,10 +1528,8 @@ struct World2 {
     const bool keep = !(cost > T(0));
     // (aref, R) -> (u, n):  u = R f - aref is -(J.qacc_warm) when the warm start is kept and -aref when it is dropped;
     // n = -1 / (1/m1 + 1/m2 + R) is what the sweep multiplies the residual with
-#if !(SG_EQ2 && SG_SLOT8)
     if (K.tm_cols) rows_to_tm(keep);
     else
-#endif
     for (int p = sl; p < D.nrow; p += LPW) {
       const int d12 = rd[p], d1 = d12 & 0xffff, d2 = (d12 >> 16) & 0xffff;
       T ar, R; ld2(row2 + 2 * p, ar, R);
@@ -1652,11 +1609,7 @@ struct World2 {
     const T* jg = x.jg; const T* w1 = x.w1; const T* w2 = x.w2; const T* Aw = x.Aw; const T* w3 = x.w3;
     const T A00 = Aw[0], A01 = Aw[1], A02 = Aw[2], A11 = Aw[3], A12 = Aw[4], A22 = Aw[5];
     const T R0 = w2[3], R1 = R0 * C.inv_impratio;
-#if SG_SLOT8
-    const T iwe = e >= 0 ? iwu : T(0);                   // 1 / m of the contact's slider: one value for the whole shell (SG_SLOT8)
-#else
-    const T iwe = e >= 0 ? stiw(e) : T(0);               // 1 / m of the contact's slider (CTA-shared table)
-#endif
+    const T iwe = e >= 0 ? iwu : T(0);                   // 1 / m of the contact's slider: one value for the whole shell
     const T old0 = w3[0], old1 = w3[1], old2 = w3[2];
     T la = w3[3];
     T res[3];
@@ -1690,12 +1643,11 @@ struct World2 {
       if (f0 < T(SG_MINVAL)) { f1 = 0; f2 = 0; la = 0; }
       else friction(f1, f2, la, A11, A12, A22, Aw[6], w1[3], Aw[7], bc, frc, f0);
     }
-#if SG_MV_EARLY
-    // the chain's M^-1 block on its way (shared memory) while the cost test runs
+    // the chain's M^-1 block on its way (shared memory) while the cost test runs: 1.447e7 -> 1.474e7 world-steps/s against
+    // loading it after the test (profiles/r02zc_sweep.log)
     T m16[16];
 #pragma unroll
     for (int ii = 0; ii < MAXCD; ii++) ld4(mv + 4 * ii, m16 + 4 * ii);
-#endif
 #if defined(SG_FRIC_STATS) && !defined(__CUDA_ARCH__)
     {
       // development statistics under the emulator: how many blocks are no-ops (an inactive contact that stays inactive)
@@ -1722,11 +1674,7 @@ struct World2 {
     for (int jj = 0; jj < MAXCD; jj++) gv[jj] = jg[jj] * d0f + jg[4 + jj] * d1f + jg[8 + jj] * d2f;
 #pragma unroll
     for (int ii = 0; ii < MAXCD; ii++) {
-#if SG_MV_EARLY
       const T* m4 = m16 + 4 * ii;
-#else
-      T m4[4]; ld4(mv + 4 * ii, m4);
-#endif
       ag[ii] += m4[0] * gv[0] + m4[1] * gv[1] + m4[2] * gv[2] + m4[3] * gv[3];
     }
     return change;
@@ -1738,7 +1686,7 @@ struct World2 {
     const T* mv;            // the chain's M^-1 block (shared memory)
     T* asl;                 // the world's slider accelerations (shared memory): a() + nfd
     T frc;                  // contact friction coefficient
-    T iwu;                  // 1 / slider mass of a uniform shell (SG_SLOT8)
+    T iwu;                  // 1 / slider mass (uniform shell)
     int lmask, mystart, mycnt;
     bool chain_lane;
     bool primed;            // ring mode: the first record of the next sweep is already on its way
@@ -1841,13 +1789,8 @@ struct World2 {
             if (k + 1 < cnt) cp_rec<RB>(ring + ((k + 1) & 1) * RB, recb + (size_t)((unsigned)(entB & 0xff) * RB));
           }
           k++;
-          if (!RING) {
-#if SG_PF_DIST == 1
-            if (k < cnt) prefetch_l1(recb + (size_t)((unsigned)(entB & 0xff) * RB));       // the next block's record
-#else
-            if (k + 1 < cnt) prefetch_l1(recb + (size_t)((unsigned)(entC & 0xff) * RB));   // two blocks ahead, as the entries
-#endif
-          }
+          // two blocks ahead, as the entries (one block ahead measures the same, profiles/r02o_sweep.log: 1.216e7 / 1.223e7)
+          if (!RING && k + 1 < cnt) prefetch_l1(recb + (size_t)((unsigned)(entC & 0xff) * RB));
           const int entD = (k + 2 < cnt) ? order[k + 2] : 0;
           impr -= contact_block<RING>(r, rl, e, cs.ag, cs.mv, cs.asl, cs.frc, cs.iwu);
           entA = entB; entB = entC; entC = entD;
@@ -1877,64 +1820,6 @@ struct World2 {
   // Per row the sweep keeps (u, n) with u = R f - aref and n = -1 / (1/m1 + 1/m2 + R): the residual is a1 - a2 + u, the
   // force change dl = res * n, and since an (unclamped) equality row has zero residual right after its own update, the
   // new u is simply a2' - a1' -- neither R nor f is needed, and there is no division in the sweep.
-#if SG_EQ2 && SG_SLOT8
-  // Two rows per lane and step: row A, then row B on the same lane -- B is either the successor of A on its dependency chain
-  // (the shared slider's new acceleration is handed over in a register: flag bits 26..29 of yb) or an independent row.
-  // All shared-memory operands of both rows are loaded up front; A's stores precede B's, so a slider both rows update ends
-  // with B's value.  Half the steps of the one-row sweep, i.e. half the load -> flops -> store -> barrier latencies.
-  template <bool GATED>
-  __device__ __forceinline__ T equality_rows(bool done) {
-    const int nstep = D.nstep;
-    char* avb = reinterpret_cast<char*>(a() + D.nfd);
-    char* rwb = reinterpret_cast<char*>(hot);
-    T acc = 0;
-    const T iwu = stim[0];
-    Slot<T> sn = ld_slot<T>(slots);
-#pragma unroll 2
-    for (int st = 0; st < nstep; st++) {
-      const Slot<T> sc = sn;
-      sn = ld_slot<T>(slots + (st + 1) * LPW);
-      const unsigned oa2 = sc.x >> 16, ob2 = sc.xb >> 16;
-      const bool va = (sc.y & 0x40000000u) != 0u, ha2 = oa2 != 0xffffu;
-      const bool vb = (sc.yb & 0x40000000u) != 0u, hb2 = ob2 != 0xffffu;
-      T* pa1 = reinterpret_cast<T*>(avb + (sc.x & 0xffffu));
-      T* pa2 = reinterpret_cast<T*>(avb + oa2);
-      T* pra = reinterpret_cast<T*>(rwb + (sc.y & 0x3ffffffu));
-      T* pb1 = reinterpret_cast<T*>(avb + (sc.xb & 0xffffu));
-      T* pb2 = reinterpret_cast<T*>(avb + ob2);
-      T* prb = reinterpret_cast<T*>(rwb + (sc.yb & 0x3ffffffu));
-      T a1 = 0, a2 = 0, u = 0, n = 0, b1 = 0, b2 = 0, ub = 0, nb = 0;
-      if (va) { a1 = *pa1; ld2(pra, u, n); }
-      if (ha2) a2 = *pa2;
-      if (vb) { ld2(prb, ub, nb); if (!(sc.yb & 0x0c000000u)) b1 = *pb1; }
-      if (hb2 && !(sc.yb & 0x30000000u)) b2 = *pb2;
-      // row A
-      const T res = (a1 - a2) + u;
-      if (GATED) n = done ? T(0) : n;
-      const T dl = res * n;
-      acc += dl * res;
-      a1 += iwu * dl; a2 -= (ha2 ? iwu : T(0)) * dl;
-      T un = a2 - a1;
-      if (GATED) un = done ? u : un;
-      // row B, with A's results where the rows share a slider
-      b1 = (sc.yb & 0x04000000u) ? a1 : b1; b1 = (sc.yb & 0x08000000u) ? a2 : b1;
-      b2 = (sc.yb & 0x10000000u) ? a1 : b2; b2 = (sc.yb & 0x20000000u) ? a2 : b2;
-      const T resb = (b1 - b2) + ub;
-      if (GATED) nb = done ? T(0) : nb;
-      const T dlb = resb * nb;
-      acc += dlb * resb;
-      b1 += iwu * dlb; b2 -= (hb2 ? iwu : T(0)) * dlb;
-      T unb = b2 - b1;
-      if (GATED) unb = done ? ub : unb;
-      if (va) { *pra = un; *pa1 = a1; }
-      if (ha2) *pa2 = a2;
-      if (vb) { *prb = unb; *pb1 = b1; }
-      if (hb2) *pb2 = b2;
-      __syncwarp();
-    }
-    return T(-0.5) * acc;
-  }
-#else
   // TM: the (u, n) pair of this lane's slot of step `st` is in the lane's tensor memory at column st * TmPair<T>::cols
   // (written by rows_to_tm at the end of the warm start); the pair of the next step is requested before this step's
   // arithmetic, so the sweep never waits for it.  Padding slots hold (0, 0) and go through the arithmetic as zeros.
@@ -1948,18 +1833,12 @@ struct World2 {
     unsigned tcol = tm;
     T un_ = 0, nn_ = 0;
     if (TM) tm_ld2(tcol, un_, nn_);
-#if SG_SLOT8
     const T iwu = stim[0];                       // 1 / element mass, the same for every slider
-#endif
     // one row per lane per step, a warp barrier where the schedule asks for one.  The next step's slot is fetched
     // before the barrier so that its latency overlaps this step's arithmetic.
     Slot<T> sn = ld_slot<T>(slots);
-#ifndef SG_EQ_UNROLL
-#define SG_EQ_UNROLL 4   // measured: 1.202e7 / 1.200e7 / 1.227e7 world-steps/s at 1 / 2 / 4 (profiles/r02j_sweep.log)
-#endif
-#define SG_PRAGMA_(x) _Pragma(#x)
-#define SG_PRAGMA(x) SG_PRAGMA_(x)
-    SG_PRAGMA(unroll SG_EQ_UNROLL)
+    // unrolled by four: 1.202e7 / 1.200e7 / 1.227e7 world-steps/s at 1 / 2 / 4 (profiles/r02j_sweep.log)
+#pragma unroll 4
     for (int st = 0; st < nstep; st++) {
       const Slot<T> sc = sn;
       sn = ld_slot<T>(slots + (st + 1) * LPW);   // the table carries one empty step past the end
@@ -1980,11 +1859,7 @@ struct World2 {
       if (GATED) n = done ? T(0) : n;
       const T dl = res * n;
       acc += dl * res;
-#if SG_SLOT8
       a1 += iwu * dl; a2 -= (has2 ? iwu : T(0)) * dl;        // fix rows have no second slider
-#else
-      a1 += sc.iw1 * dl; a2 -= sc.iw2 * dl;
-#endif
       T un = a2 - a1;
       if (GATED) un = done ? u : un;
       if (TM) { tm_st1(tcol, un); tcol += CW; if (valid) *pa1 = a1; }
@@ -2005,9 +1880,7 @@ struct World2 {
     const char* rwb = reinterpret_cast<const char*>(hot);
     constexpr unsigned CW = TmPair<T>::cols;
     unsigned tcol = tm;
-#if SG_SLOT8
     const T iwu = stim[0];
-#endif
     for (int st = 0; st <= nstep; st++, tcol += CW) {
       const Slot<T> sc = ld_slot<T>(slots + st * LPW);
       const unsigned o2 = sc.x >> 16;
@@ -2016,13 +1889,8 @@ struct World2 {
       if (valid) {
         T ar, R; ld2(reinterpret_cast<const T*>(rwb + (sc.y & 0x3fffffffu)), ar, R);
         T ja = *reinterpret_cast<const T*>(avb + (sc.x & 0xffffu));
-#if SG_SLOT8
         T diag = iwu;
         if (has2) { ja -= *reinterpret_cast<const T*>(avb + o2); diag += iwu; }
-#else
-        T diag = sc.iw1;
-        if (has2) { ja -= *reinterpret_cast<const T*>(avb + o2); diag += sc.iw2; }
-#endif
         u = keep ? -ja : -ar;
         n = T(-1) / (diag + R);
       }
@@ -2041,40 +1909,27 @@ struct World2 {
     }
     __syncwarp();
   }
-#endif
   __device__ __forceinline__ T equality_sweep(Tendon& tn, bool done) {
     const int ns = D.ns;
     T* av = a() + D.nfd;
     // worlds stop sweeping one by one (rarely before the last sweep): the gated loop is only taken by a warp that
     // holds a finished world
-#if SG_EQ2 && SG_SLOT8
-    T impr = __any_sync(FULLMASK, done) ? equality_rows<true>(done) : equality_rows<false>(false);
-#else
     T impr;
     if (K.tm_cols) impr = __any_sync(FULLMASK, done) ? equality_rows<true, true>(done) : equality_rows<false, true>(false);
     else impr = __any_sync(FULLMASK, done) ? equality_rows<true>(done) : equality_rows<false>(false);
-#endif
     // volume-tendon row: dense over the shell, sub-warp shuffle reduction
     {
       T s = 0;
-#if SG_SLOT8
 #pragma unroll 4
       for (int e = sl; e < ns; e += LPW) s += av[e];            // tendon coefficients are all 1
-#else
-      for (int e = sl; e < ns; e += LPW) s += stc[e] * av[e];
-#endif
       s = gsum(s);
       const T res = s + tn.u;
       const T dl = done ? T(0) : res * tn.nA;
       if (sl == 0) impr -= T(0.5) * dl * res;
       tn.u += tn.R * dl;
-#if SG_SLOT8
       const T da = stim[0] * dl;
 #pragma unroll 4
       for (int e = sl; e < ns; e += LPW) av[e] += da;
-#else
-      for (int e = sl; e < ns; e += LPW) av[e] += stciw[e] * dl;
-#endif
       __syncwarp();
     }
     return impr;
@@ -2149,9 +2004,7 @@ struct World2 {
     }
     __syncwarp();
     tick(PH_SENSORS);
-#if !(SG_EQ2 && SG_SLOT8)
     if (K.tm_cols && K.debug_out && __any_sync(FULLMASK, valid && w == K.debug_world)) rows_from_tm();
-#endif
     if (valid && w == K.debug_world) debug_dump(tn);
     bool badacc = false;
     for (int i = sl; i < D.nv; i += LPW) if (!(tabs(a()[i]) <= T(SG_MAXVAL))) badacc = true;
@@ -2294,19 +2147,11 @@ __global__ void __launch_bounds__(32 * SG_MAX_WARPS, SG_MIN_CTAS) sg_step_kernel
   }
 #endif
   {
-    // stage the step tables: one {descriptor, (1/m, 1/m)} slot per (step, lane)
+    // stage the step tables: one descriptor slot per (step, lane)
     Slot<T>* ss = reinterpret_cast<Slot<T>*>(smem_raw);
     const int nslot = (D.nstep + 1) * LPW;
     for (int i = threadIdx.x; i < nslot; i += blockDim.x) {
-#if SG_EQ2 && SG_SLOT8
-      Slot<T> t; t.x = (unsigned)K.itab[D.io_step_d + 4 * i]; t.y = (unsigned)K.itab[D.io_step_d + 4 * i + 1];
-      t.xb = (unsigned)K.itab[D.io_step_d + 4 * i + 2]; t.yb = (unsigned)K.itab[D.io_step_d + 4 * i + 3];
-#else
       Slot<T> t; t.x = (unsigned)K.itab[D.io_step_d + 2 * i]; t.y = (unsigned)K.itab[D.io_step_d + 2 * i + 1];
-#endif
-#if !SG_SLOT8
-      t.iw1 = K.tab[D.o_step_iw + 2 * i]; t.iw2 = K.tab[D.o_step_iw + 2 * i + 1];
-#endif
       ss[i] = t;
     }
     T* tc = reinterpret_cast<T*>(smem_raw + (size_t)nslot * sizeof(Slot<T>));

@@ -6,13 +6,6 @@
 // It replaces what mj_loadXML/mj_makeData hand to mj_step in the reference (ref: environment/manenv.py:27-28).
 // Anything outside that model family is rejected with an error -- there is no generic/CPU fallback.
 #pragma once
-// two equality rows per lane and step (see build_step_tables2); needs SG_SLOT8.  Measured (profiles/r02l_sweep.log): 31 fused
-// steps instead of 58 for softbox, bit-identical results, but 1.199e7 against 1.224e7 world-steps/s -- at 16 warps per SM the
-// equality sweep is bound by shared-memory wavefronts (ncu: ~26 000 per warp-step, 19 % of them bank conflicts), which
-// fusing does not reduce, not by the latency of a step.  Off; kept as an A/B switch and for low-occupancy launches.
-#ifndef SG_EQ2
-#define SG_EQ2 0
-#endif
 #include <algorithm>
 #include <cmath>
 #include <cstdint>
@@ -79,7 +72,7 @@ struct PlanDims {
   int io_run, nrun; // broadphase runs of the pair list: {pair type, first collider | colliders << 8, first second geom, count}
   // per-batch step tables of the level sweep (depend on the lanes per world; appended by sg_api.cu)
   int io_step_d;    // 2*(nstep+1)*lpw ints: {byte offset of d1 | of d2 << 16, byte offset of the row pair | barrier << 31} per slot
-  int o_step_iw;    // 2*nstep*lpw reals: {1/m first, 1/m second} per slot
+  int o_step_iw;    // unused: the slots carry no masses (every shell slider has the same one)
   int nstep;
 };
 
@@ -163,10 +156,13 @@ struct Plan {
 // arrays) is chosen so that the rows of a step get distinct residues.  Padding slots and the missing second slider of
 // fix rows are predicated off by the kernel (second-slider offset 0xffff, valid bit clear).
 // Slot encoding (esize = bytes per real of the kernel precision): {first slider * esize | second slider * esize << 16,
-// row position * 2 * esize | valid << 30 | barrier << 31}, {1/m first, 1/m second}.
-inline int build_step_tables_for(const PlanDims& D, const std::vector<double>& tab, const std::vector<int>& itab, int lpw, int esize,
-                                 int target, std::vector<int>& step_d, std::vector<double>& step_iw, std::vector<int>& perm) {
-  step_d.clear(); step_iw.clear();
+// row position * 2 * esize | valid << 30 | barrier << 31}.
+// (A second scheduler that gave every lane two rows per step -- 31 steps instead of 58 for softbox, bit-identical results --
+// measured 2 % slower, profiles/r02l_sweep.log: at 16 warps per SM the sweep is bound by shared-memory wavefronts, which
+// fusing does not reduce, not by the latency of a step.  It was removed.)
+inline int build_step_tables_for(const PlanDims& D, const std::vector<int>& itab, int lpw, int esize, int target,
+                                 std::vector<int>& step_d, std::vector<int>& perm) {
+  step_d.clear();
   const int nrow = D.nrow;
   const bool avoid = target > 0;
   const int R = lpw < 32 ? lpw : 32;                 // residue modulus: bank distance of the worlds of a warp
@@ -240,16 +236,14 @@ inline int build_step_tables_for(const PlanDims& D, const std::vector<double>& t
     }
   } else for (int p = 0; p < nrow; p++) perm[p] = p;
   auto emit = [&](int p, int fl) {
-    unsigned x = 0xffffffffu, y = (unsigned)fl << 31; double iw1 = 0, iw2 = 0;
+    unsigned x = 0xffffffffu, y = (unsigned)fl << 31;
     if (p >= 0) {
       const int d1 = itab[D.io_row_d1 + p], d2 = itab[D.io_row_d2 + p];
-      iw1 = 1.0 / tab[D.o_sl_m + d1];
-      unsigned o2 = 0xffffu;
-      if (d2 >= 0) { o2 = (unsigned)(d2 * esize); iw2 = 1.0 / tab[D.o_sl_m + d2]; }
+      const unsigned o2 = d2 >= 0 ? (unsigned)(d2 * esize) : 0xffffu;
       x = (unsigned)(d1 * esize) | (o2 << 16);
       y = ((unsigned)fl << 31) | (unsigned)(perm[p] * 2 * esize) | (1u << 30);
     }
-    step_d.push_back((int)x); step_d.push_back((int)y); step_iw.push_back(iw1); step_iw.push_back(iw2);
+    step_d.push_back((int)x); step_d.push_back((int)y);
   };
   for (int s = 0; s < nstep; s++) for (int k = 0; k < lpw; k++) emit(k < (int)steps[s].size() ? steps[s][k] : -1, flag[s]);
   // one empty step past the end: the sweep prefetches the next step's descriptors unconditionally
@@ -291,203 +285,20 @@ inline long sweep_wavefronts(const std::vector<int>& step_d, int lpw, int esize)
   return total;
 }
 
-// ---- two rows per lane and step (SG_EQ2) ---------------------------------------------------------------------------
-// The equality sweep is bound by the latency of one step (shared-memory load -> five dependent flops -> store -> warp
-// barrier, ~130 cycles) times the number of steps, and the dependency chains of the composite alternate fix rows and
-// neighbour rows that share a slider: fix(i) -> nb(i, j) -> fix(j) -> nb(j, k) ...  A lane therefore takes TWO rows per step:
-// row A as before, and a row B that is either the successor of its own A on that chain (the shared slider's new
-// acceleration is handed over in a register, flags below) or any other row that is ready and independent of every
-// other lane's rows of the step.  Row B runs after row A on the same lane, different lanes never share a slider within a
-// step, and rows that share a slider keep MuJoCo's order: the result is that of the sequential sweep, in about half
-// the steps (softbox: 53 -> 28 + slack).
-// Slot encoding, four words per (step, lane): {xA, yA, xB, yB}; x = first slider * esize | second slider * esize << 16
-// (0xffff: none); y = row position * 2 * esize (bits 0..25) | valid << 30; yB also carries the hand-over flags: bit 26 /
-// 27: B's FIRST slider is A's first / second slider, bit 28 / 29: B's SECOND slider is A's first / second slider.
-inline int build_step_tables2_for(const PlanDims& D, const std::vector<int>& itab, int lpw, int esize, int target,
-                                  std::vector<int>& step_d, std::vector<int>& perm) {
-  step_d.clear();
-  const int nrow = D.nrow;
-  const bool avoid = target > 0;
-  const int R = lpw < 32 ? lpw : 32;
-  SG_REQUIRE((size_t)(D.ns + 1) * esize < 0xffff && (size_t)(nrow + 1) * 2 * esize < (1u << 26), "too many shell joints for the packed step descriptors");
-  std::vector<int> last(D.ns, -1), height(nrow, 1), step_of(nrow, -1);
-  std::vector<std::vector<int>> pred(nrow), succ(nrow);
-  for (int p = 0; p < nrow; p++) {
-    const int ds[2] = {itab[D.io_row_d1 + p], itab[D.io_row_d2 + p]};
-    for (int k = 0; k < 2; k++) {
-      const int d = ds[k];
-      if (d < 0) continue;
-      const int q = last[d];
-      if (q >= 0 && (pred[p].empty() || pred[p].back() != q)) { pred[p].push_back(q); succ[q].push_back(p); }
-      last[d] = p;
-    }
-  }
-  for (int p = nrow - 1; p >= 0; p--) for (int s : succ[p]) if (height[s] + 1 > height[p]) height[p] = height[s] + 1;
-  // with two chained rows per step the critical path shrinks to about half: slack is counted in fused steps
-  auto fused_height = [&](int p) { return (height[p] + 1) / 2; };
-  std::vector<char> done(nrow, 0), sched(nrow, 0);
-  struct Pair { int a, b; };
-  std::vector<std::vector<Pair>> steps;
-  int ndone = 0;
-  auto sliders = [&](int p, int* d) { d[0] = itab[D.io_row_d1 + p]; d[1] = itab[D.io_row_d2 + p]; };
-  while (ndone < nrow) {
-    const int now = (int)steps.size();
-    std::vector<int> ready;
-    for (int p = 0; p < nrow; p++) {
-      if (sched[p]) continue;
-      bool ok = true;
-      for (int q : pred[p]) if (!done[q]) { ok = false; break; }
-      if (ok) ready.push_back(p);
-    }
-    SG_REQUIRE(!ready.empty(), "cyclic equality schedule");
-    std::stable_sort(ready.begin(), ready.end(), [&](int a, int b) { return height[a] != height[b] ? height[a] > height[b] : a < b; });
-    std::vector<Pair> cur;
-    std::vector<char> use1(R, 0), use2(R, 0), useB1(R, 0), useB2(R, 0);
-    std::vector<char> used(D.ns, 0);
-    for (int p : ready) {
-      if ((int)cur.size() >= lpw) break;
-      int d[2]; sliders(p, d);
-      const bool clash = avoid && (use1[d[0] % R] || (d[1] >= 0 && use2[d[1] % R]));
-      const bool must = now + fused_height(p) >= target;
-      if (clash && !must) continue;
-      cur.push_back({p, -1}); sched[p] = 1; use1[d[0] % R] = 1; used[d[0]] = 1;
-      if (d[1] >= 0) { use2[d[1] % R] = 1; used[d[1]] = 1; }
-    }
-    // second rows: the best row (by remaining chain length) whose predecessors are done or are this lane's own row A and
-    // whose sliders are not touched by any other lane in this step
-    for (size_t k = 0; k < cur.size(); k++) {
-      const int pa = cur[k].a;
-      int da[2]; sliders(pa, da);
-      int best = -1;
-      for (int pass = 0; pass < 2 && best < 0; pass++)        // pass 0: conflict-free positions only
-        for (int q = 0; q < nrow; q++) {
-          if (sched[q]) continue;
-          bool ok = true;
-          for (int x : pred[q]) if (!done[x] && x != pa) { ok = false; break; }
-          if (!ok) continue;
-          int dq[2]; sliders(q, dq);
-          bool indep = true;
-          for (int i = 0; i < 2; i++) if (dq[i] >= 0 && used[dq[i]] && dq[i] != da[0] && dq[i] != da[1]) indep = false;
-          if (!indep) continue;
-          if (pass == 0 && avoid && (useB1[dq[0] % R] || (dq[1] >= 0 && useB2[dq[1] % R]))) continue;
-          if (best < 0 || height[q] > height[best]) best = q;
-        }
-      if (best >= 0) {
-        int dq[2]; sliders(best, dq);
-        cur[k].b = best; sched[best] = 1; useB1[dq[0] % R] = 1; used[dq[0]] = 1;
-        if (dq[1] >= 0) { useB2[dq[1] % R] = 1; used[dq[1]] = 1; }
-      }
-    }
-    for (const Pair& pr : cur) { done[pr.a] = 1; step_of[pr.a] = now; ndone++; if (pr.b >= 0) { done[pr.b] = 1; step_of[pr.b] = now; ndone++; } }
-    steps.push_back(cur);
-  }
-  const int nstep = (int)steps.size();
-  // storage positions: the A rows of a step get distinct residues, and so do its B rows (two separate 64-bit loads)
-  perm.assign(nrow, -1);
-  if (avoid) {
-    std::vector<int> cap(R, 0), usedr(R, 0);
-    for (int q = 0; q < nrow; q++) cap[q % R]++;
-    auto place = [&](int p, std::vector<char>& taken) {
-      int best = -1;
-      for (int pass = 0; pass < 2 && best < 0; pass++)
-        for (int r = 0; r < R; r++) {
-          if (usedr[r] >= cap[r] || (pass == 0 && taken[r])) continue;
-          if (best < 0 || cap[r] - usedr[r] > cap[best] - usedr[best]) best = r;
-        }
-      SG_REQUIRE(best >= 0, "row storage assignment");
-      taken[best] = 1;
-      perm[p] = best + R * usedr[best]++;
-    };
-    for (int s = 0; s < nstep; s++) {
-      std::vector<char> takenA(R, 0), takenB(R, 0);
-      for (const Pair& pr : steps[s]) place(pr.a, takenA);
-      for (const Pair& pr : steps[s]) if (pr.b >= 0) place(pr.b, takenB);
-    }
-  } else for (int p = 0; p < nrow; p++) perm[p] = p;
-  auto enc = [&](int p, unsigned& x, unsigned& y) {
-    x = 0xffffffffu; y = 0;
-    if (p < 0) return;
-    const int d1 = itab[D.io_row_d1 + p], d2 = itab[D.io_row_d2 + p];
-    x = (unsigned)(d1 * esize) | ((d2 >= 0 ? (unsigned)(d2 * esize) : 0xffffu) << 16);
-    y = (unsigned)(perm[p] * 2 * esize) | (1u << 30);
-  };
-  auto emit = [&](int pa, int pb) {
-    unsigned xa, ya, xb, yb;
-    enc(pa, xa, ya); enc(pb, xb, yb);
-    if (pa >= 0 && pb >= 0) {
-      const int a1 = itab[D.io_row_d1 + pa], a2 = itab[D.io_row_d2 + pa], b1 = itab[D.io_row_d1 + pb], b2 = itab[D.io_row_d2 + pb];
-      if (b1 == a1) yb |= 1u << 26; else if (a2 >= 0 && b1 == a2) yb |= 1u << 27;
-      if (b2 >= 0) { if (b2 == a1) yb |= 1u << 28; else if (a2 >= 0 && b2 == a2) yb |= 1u << 29; }
-    }
-    step_d.push_back((int)xa); step_d.push_back((int)ya); step_d.push_back((int)xb); step_d.push_back((int)yb);
-  };
-  for (int s = 0; s < nstep; s++)
-    for (int k = 0; k < lpw; k++) { if (k < (int)steps[s].size()) emit(steps[s][k].a, steps[s][k].b); else emit(-1, -1); }
-  for (int k = 0; k < lpw; k++) emit(-1, -1);      // one empty step past the end (descriptor prefetch)
-  return nstep;
-}
-
-// shared-memory wavefronts of one fused sweep (same model as sweep_wavefronts, A and B rows are separate accesses)
-inline long sweep_wavefronts2(const std::vector<int>& step_d, int lpw, int esize) {
-  (void)esize;
-  const int wpw = 32 / lpw, nslot = (int)step_d.size() / 4, nstep = nslot / lpw - 1;
-  long total = 0;
-  auto worst_bank = [&](const std::vector<long>& word) {
-    int worst = 0;
-    for (int b = 0; b < 32; b++) {
-      std::vector<long> seen;
-      for (long w : word) { if (w < 0) continue; if (w % 32 == b && std::find(seen.begin(), seen.end(), w) == seen.end()) seen.push_back(w); }
-      worst = std::max(worst, (int)seen.size());
-    }
-    return worst;
-  };
-  for (int s = 0; s < nstep; s++)
-    for (int half = 0; half < 2; half++) {
-      std::vector<long> a1, a2, rw;
-      for (int g = 0; g < wpw; g++) {
-        const int slot = wpw > 1 ? (g % (wpw / 2)) * 2 + g / (wpw / 2) : 0;
-        for (int k = 0; k < lpw; k++) {
-          const unsigned x = (unsigned)step_d[4 * (s * lpw + k) + 2 * half], y = (unsigned)step_d[4 * (s * lpw + k) + 2 * half + 1];
-          const long goff = (long)slot * lpw + 4096L * slot;
-          const bool valid = (y >> 30) & 1, has2 = (x >> 16) != 0xffffu;
-          a1.push_back(valid ? goff + (x & 0xffff) / 4 : -1); a2.push_back(valid && has2 ? goff + (x >> 16) / 4 : -1);
-          rw.push_back(valid ? goff + (y & 0x3ffffffu) / 4 : -1);
-        }
-      }
-      total += 2 * worst_bank(a1) + 2 * worst_bank(a2) + worst_bank(rw);
-    }
-  return total;
-}
-
-inline void build_step_tables2(const PlanDims& D, const std::vector<int>& itab, int lpw, int esize, std::vector<int>& step_d,
-                               std::vector<int>& perm, bool avoid_conflicts = true) {
-  const int base = build_step_tables2_for(D, itab, lpw, esize, 0, step_d, perm);
-  if (!avoid_conflicts) return;
-  const double per_step = 10.0;                      // fixed cost of a fused step (issue, barrier) in wavefront units
-  double best_cost = 1e300; int best_target = 0;
-  for (int target = base; target <= base + base / 4 + 4; target++) {
-    std::vector<int> sd, pm;
-    const int n = build_step_tables2_for(D, itab, lpw, esize, target, sd, pm);
-    const double cost = (double)sweep_wavefronts2(sd, lpw, esize) + per_step * n;
-    if (cost < best_cost) { best_cost = cost; best_target = target; }
-  }
-  build_step_tables2_for(D, itab, lpw, esize, best_target, step_d, perm);
-}
-
 // the schedule the kernel runs: the target length (critical path + slack) with the least estimated cost
-inline void build_step_tables(const PlanDims& D, const std::vector<double>& tab, const std::vector<int>& itab, int lpw, int esize,
-                              std::vector<int>& step_d, std::vector<double>& step_iw, std::vector<int>& perm, bool avoid_conflicts = true) {
-  const int base = build_step_tables_for(D, tab, itab, lpw, esize, 0, step_d, step_iw, perm);
+inline void build_step_tables(const PlanDims& D, const std::vector<int>& itab, int lpw, int esize, std::vector<int>& step_d,
+                              std::vector<int>& perm, bool avoid_conflicts = true) {
+  const int base = build_step_tables_for(D, itab, lpw, esize, 0, step_d, perm);
   if (!avoid_conflicts) return;
   const double per_step = 6.0;                       // fixed cost of a step (issue, barrier) in wavefront units
   double best_cost = 1e300; int best_target = 0;
   for (int target = base; target <= base + base / 4 + 4; target++) {
-    std::vector<int> sd, pm; std::vector<double> si;
-    const int n = build_step_tables_for(D, tab, itab, lpw, esize, target, sd, si, pm);
+    std::vector<int> sd, pm;
+    const int n = build_step_tables_for(D, itab, lpw, esize, target, sd, pm);
     const double cost = (double)sweep_wavefronts(sd, lpw, esize) + per_step * n;
     if (cost < best_cost) { best_cost = cost; best_target = target; }
   }
-  build_step_tables_for(D, tab, itab, lpw, esize, best_target, step_d, step_iw, perm);
+  build_step_tables_for(D, itab, lpw, esize, best_target, step_d, perm);
 }
 
 inline bool same(const double* a, const double* b, int n) { for (int i = 0; i < n; i++) if (a[i] != b[i]) return false; return true; }

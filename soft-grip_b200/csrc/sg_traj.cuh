@@ -56,9 +56,9 @@ __device__ __forceinline__ float u01(uint32_t x) { return (float)x * 2.328306436
 //   * the angle is taken in (-pi, pi] (cos and sin of 2 pi u are minus those of 2 pi (u - 0.5), and u - 0.5 is exact above
 //     0.25), where sin.approx / cos.approx are good to 2^-20.9 absolute.
 // About 50 instructions per pair instead of ~170 with the FFMA polynomials of logf / sincospif: the kernel is bound by
-// HBM instead of by issue slots (DESIGN.md 3b).  -DSG_TRAJ_ACCURATE_NORMALS keeps the libdevice version for A/B runs.
+// HBM instead of by issue slots (DESIGN.md 3b).  The host build (the SIMT emulator of the tests) keeps the libm formulas.
 __device__ __forceinline__ void box_muller(uint32_t a, uint32_t b, float& z0, float& z1) {
-#if defined(SG_TRAJ_ACCURATE_NORMALS) || !defined(__CUDA_ARCH__)
+#if !defined(__CUDA_ARCH__)
   const float r = sqrtf(-2.0f * logf(u01(a)));
   float s, c;
   sincospif(2.0f * u01(b), &s, &c);

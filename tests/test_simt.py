@@ -36,10 +36,10 @@ def states():
     return np.load(os.path.join(GOLDEN, "softbox_states.npz"))
 
 
-@pytest.mark.parametrize("prec,lpw,aux", [(64, 8, 0), (64, 4, 0), (64, 32, 0), (64, 16, 0), (32, 8, 0)])
-def test_emulated_single_step_parity_against_golden_states(emu, states, prec, lpw, aux):
+@pytest.mark.parametrize("prec,lpw", [(64, 8), (64, 4), (64, 32), (64, 16), (32, 8)])
+def test_emulated_single_step_parity_against_golden_states(emu, states, prec, lpw):
     W = 32 // lpw + 1                      # one full warp of worlds plus a ragged tail
-    env = emu.EmuBatch(blob_path("softbox"), W, prec=prec, lpw=lpw, aux_smem=aux)
+    env = emu.EmuBatch(blob_path("softbox"), W, prec=prec, lpw=lpw)
     env.set_params(stiffness=np.full(W, 700.0))
     env.set_debug_world(W - 1)
     idx = range(len(states["step"])) if (prec, lpw) == (64, 8) else range(0, len(states["step"]), 3)
@@ -301,7 +301,7 @@ def test_emulated_other_models_first_steps(emu, make_world, name):
 
 
 def _decode_schedule(env):
-    """-> nstep, lanes, bytes per real, nrow, modelled wavefronts, rows per slot (1 or 2), slots [nstep+1][lanes][2*rps], perm."""
+    """-> nstep, lanes, bytes per real, nrow, modelled wavefronts, rows per slot, slots [nstep+1][lanes][2*rps], perm."""
     t = env.debug("sweep_schedule")
     nstep, lpw, esize, nrow = (int(x) for x in t[:4])
     rps = int(t[4] // 1e9)
@@ -315,16 +315,16 @@ def _decode_schedule(env):
 @pytest.mark.parametrize("model,lpw,prec", [("softbox", 8, 32), ("softbox", 4, 32), ("softbox", 16, 64), ("softball", 8, 32), ("softcylinder", 8, 64),
                                             ("softbox_refined", 32, 32)])
 def test_equality_sweep_schedule_is_a_valid_gauss_seidel_order(emu, model, lpw, prec):
-    """Host logic of the equality sweep (sg_plan.hpp build_step_tables / build_step_tables2): every row is swept exactly
-    once; within a step different lanes share no slider; a lane's second row (two rows per slot) may share sliders with its
-    own first row only, with the hand-over flags saying so; rows that share a slider keep MuJoCo's order (an earlier step,
-    or first / second row of one lane); the storage positions are a permutation; and the conflict-aware schedule costs no
-    more modelled shared-memory wavefronts than the plain list schedule."""
+    """Host logic of the equality sweep (sg_plan.hpp build_step_tables): one row per slot; every row is swept exactly
+    once; within a step different lanes share no slider; rows that share a slider keep MuJoCo's order (an earlier step);
+    the storage positions are a permutation; and the conflict-aware schedule costs no more modelled shared-memory
+    wavefronts than the plain list schedule."""
     import importlib
     mjcf = importlib.import_module("soft-grip_b200.mjcf")
     A = mjcf.load_blob(blob_path(model)).arrays
     env = emu.EmuBatch(blob_path(model), 2, prec=prec, lpw=lpw)
     nstep, lpw_, esize, nrow, wavefronts, rps, sd, perm = _decode_schedule(env)
+    assert rps == 1
     assert lpw_ == lpw and esize == prec // 8 and nrow == len(A["eq_obj1id"]) - 1
     assert sorted(perm.tolist()) == list(range(nrow))
     nfd = int((A["jnt_type"] == 3).sum())                      # hinge joints of the fingers come first
@@ -333,45 +333,33 @@ def test_equality_sweep_schedule_is_a_valid_gauss_seidel_order(emu, model, lpw, 
         d1, d2 = int(A["eq_obj1id"][r]) - nfd, int(A["eq_obj2id"][r])
         key_to_eq[(d1, d2 - nfd if d2 >= 0 else -1)] = r
     assert len(key_to_eq) == nrow
-    posmask = 0x3fffffff if rps == 1 else 0x3ffffff
-    when, seen_pos = {}, set()                                 # row -> (step, lane, half)
+    when, seen_pos = {}, set()                                 # row -> step
     for s in range(nstep):
         owner = {}                                             # slider -> lane that touches it in this step
         for k in range(lpw):
-            first = None
-            for half in range(rps):
-                x, y = int(sd[s, k, 2 * half]), int(sd[s, k, 2 * half + 1])
-                if not (y >> 30) & 1:
-                    assert half == 0 or (y >> 26) == 0
-                    continue
-                assert half == 0 or first is not None         # a second row only behind a first one
-                d1 = (x & 0xffff) // esize
-                d2 = (x >> 16) // esize if (x >> 16) != 0xffff else -1
-                pos = (y & posmask) // (2 * esize)
-                assert pos not in seen_pos and 0 <= pos < nrow
-                seen_pos.add(pos)
-                for d in (d1, d2):
-                    if d >= 0:
-                        assert owner.setdefault(d, k) == k     # different lanes of a step touch disjoint sliders
-                if half == 1:
-                    fl = (y >> 26) & 15
-                    want = (1 if d1 == first[0] else 2 if d1 == first[1] else 0) | ((4 if d2 == first[0] else 8 if d2 == first[1] else 0) if d2 >= 0 else 0)
-                    assert fl == want, (s, k, fl, want)        # the hand-over flags name exactly the shared sliders
-                else:
-                    first = (d1, d2 if d2 >= 0 else -2)
-                r = key_to_eq[(d1, d2)]
-                assert r not in when
-                when[r] = (s, k, half)
+            x, y = int(sd[s, k, 0]), int(sd[s, k, 1])
+            if not (y >> 30) & 1:
+                continue
+            d1 = (x & 0xffff) // esize
+            d2 = (x >> 16) // esize if (x >> 16) != 0xffff else -1
+            pos = (y & 0x3fffffff) // (2 * esize)
+            assert pos not in seen_pos and 0 <= pos < nrow
+            seen_pos.add(pos)
+            for d in (d1, d2):
+                if d >= 0:
+                    assert owner.setdefault(d, k) == k         # different lanes of a step touch disjoint sliders
+            r = key_to_eq[(d1, d2)]
+            assert r not in when
+            when[r] = s
     assert len(when) == nrow
-    assert all(not (int(sd[nstep, k, 2 * h + 1]) >> 30) & 1 for k in range(lpw) for h in range(rps))   # padding step
+    assert all(not (int(sd[nstep, k, 1]) >> 30) & 1 for k in range(lpw))   # padding step
     last = {}
     for r in range(nrow):                                      # MuJoCo's sequential order
         for d in (int(A["eq_obj1id"][r]) - nfd, int(A["eq_obj2id"][r]) - nfd if A["eq_obj2id"][r] >= 0 else None):
             if d is None:
                 continue
             if d in last:
-                (sq, kq, hq), (sr, kr, hr) = when[last[d]], when[r]
-                assert sq < sr or (sq == sr and kq == kr and hq < hr)
+                assert when[last[d]] < when[r]
             last[d] = r
     os.environ["SOFTGRIP_NO_BANK_SCHEDULE"] = "1"
     try:
@@ -380,14 +368,12 @@ def test_equality_sweep_schedule_is_a_valid_gauss_seidel_order(emu, model, lpw, 
     finally:
         del os.environ["SOFTGRIP_NO_BANK_SCHEDULE"]
     assert perm0.tolist() == list(range(nrow))
-    assert wavefronts + (10 if rps == 2 else 6) * nstep <= wavefronts0 + (10 if rps == 2 else 6) * nstep0
-    if rps == 2 and model == "softbox" and lpw == 8:
-        assert nstep <= 36                                     # 53 dependency levels in about half the steps
+    assert wavefronts + 6 * nstep <= wavefronts0 + 6 * nstep0
 
 
 def test_removed_placement_options_fail_loudly(emu):
-    """The shared-memory placement of the once-per-step data is gone from kernel 2: asking for it is an error, not a
-    silent fallback."""
+    """The shared-memory placement of the once-per-step data is gone from the step kernel: asking for it is an error, not
+    a silent fallback."""
     with pytest.raises(RuntimeError, match="removed"):
         emu.EmuBatch(blob_path("softbox"), 2, prec=32, lpw=8, aux_smem=1)
     with pytest.raises(RuntimeError, match="removed"):
@@ -562,7 +548,7 @@ def test_emulated_larger_models_at_more_lanes_per_world(emu, make_world, name, l
         assert rel(q1[-1], oq) < 1e-8 and rel(v1[-1], ov) < 1e-8 and rel(qacc[-1], oacc) < 1e-8
         steps[lanes] = int(env.debug("sweep_schedule")[0])
         env.close()
-    assert steps[lpw] < 0.8 * steps[8], steps        # (two rows per slot: softball 55 -> 42 steps, refined 99 -> 63 / 56)
+    assert steps[lpw] < 0.8 * steps[8], steps
 
 
 def test_emulated_step_kernel_is_clean_under_asan(tmp_path):
