@@ -435,10 +435,61 @@ __device__ __forceinline__ float trsqrt(float x) {
 #if defined(SG_FRIC_STATS) && !defined(__CUDA_ARCH__)
 static long sg_fric_evals = 0, sg_fric_calls = 0;     // development statistics under the emulator (Newton evaluations per call)
 #endif
+#if defined(SG_FRIC_DOMAIN) && !defined(__CUDA_ARCH__)
+// development statistics under the emulator (scripts/dev_fric_domain.py): the range of friction_fast's arguments that the
+// step kernel produces -- the domain tests/test_primitives.py asserts its error bounds on.  Per quantity: count, min, max
+// and a histogram in quarter decades, written as one JSON line to $SG_FRIC_DOMAIN_OUT when the process exits.
+struct FricDomain {
+  enum { F0, BKF, COND, COND_INACTIVE, WARM, NQ, NBIN = 320 };     // bins: log10 from -40 to +40
+  long n[NQ] = {}, hist[NQ][NBIN] = {};
+  double lo[NQ], hi[NQ];
+  long calls = 0, active = 0, kb0 = 0;
+  FricDomain() { for (int q = 0; q < NQ; q++) { lo[q] = 1e300; hi[q] = -1e300; } }
+  void add(int q, double x) {
+    if (!(x > 0)) return;
+    n[q]++; lo[q] = x < lo[q] ? x : lo[q]; hi[q] = x > hi[q] ? x : hi[q];
+    int b = (int)std::floor(4.0 * (std::log10(x) + 40.0)); b = b < 0 ? 0 : b >= NBIN ? NBIN - 1 : b;
+    hist[q][b]++;
+  }
+  void record(float a11, float a12, float kb, float bc0, float bc1, float f0, float la_in, float la_out) {
+    calls++;
+    if (kb == 0.0f) { kb0++; return; }
+    const double a22 = 1.0 - (double)a11, tr = (double)a11 + a22, det = (double)a11 * a22 - (double)a12 * a12;
+    const double disc = std::sqrt(std::fmax(0.0, 0.25 * tr * tr - det)), lmax = 0.5 * tr + disc, lmin = det / lmax;
+    const double cond = lmin > 0 ? lmax / lmin : 1e300;
+    add(F0, f0);
+    add(BKF, std::sqrt((double)bc0 * bc0 + (double)bc1 * bc1) * kb / f0);
+    add(COND, cond);
+    if (la_out != 0.0f) { active++; if (la_in != 0.0f) add(WARM, (double)la_in / la_out); }   // warm start over the root it settled on
+    else add(COND_INACTIVE, cond);
+  }
+  ~FricDomain() {
+    const char* path = getenv("SG_FRIC_DOMAIN_OUT");
+    FILE* f = path ? fopen(path, "a") : nullptr;
+    if (!f) return;
+    static const char* names[NQ] = {"f0", "bc_kb_over_f0", "cond", "cond_inactive", "warm_over_root"};
+    fprintf(f, "{\"calls\": %ld, \"active\": %ld, \"singular\": %ld", calls, active, kb0);
+    for (int q = 0; q < NQ; q++) {
+      fprintf(f, ", \"%s\": {\"n\": %ld, \"min\": %.6g, \"max\": %.6g, \"hist_log10_quarter\": {", names[q], n[q], lo[q], hi[q]);
+      bool first = true;
+      for (int b = 0; b < NBIN; b++) if (hist[q][b]) { fprintf(f, "%s\"%.2f\": %ld", first ? "" : ", ", b / 4.0 - 40.0, hist[q][b]); first = false; }
+      fprintf(f, "}}");
+    }
+    fprintf(f, "}\n");
+    fclose(f);
+  }
+};
+inline FricDomain sg_fric_domain;
+#endif
 __device__ __forceinline__ void friction_fast(float& f1, float& f2, float& la_io, float a11, float a12, float kb, float bc0, float bc1, float frc, float f0) {
 #if defined(SG_FRIC_STATS) && !defined(__CUDA_ARCH__)
   sg_fric_calls++;
   if ((sg_fric_calls & 0x3ffff) == 0) fprintf(stderr, "friction_fast: %ld calls, %.3f evaluations per call\n", sg_fric_calls, (double)sg_fric_evals / (double)sg_fric_calls);
+#endif
+#if defined(SG_FRIC_DOMAIN) && !defined(__CUDA_ARCH__)
+  // recorded on every return, with the multiplier the call settled on
+  struct Rec { float* la; float a11, a12, kb, bc0, bc1, f0, la_in; ~Rec() { sg_fric_domain.record(a11, a12, kb, bc0, bc1, f0, la_in, *la); } }
+      rec_{&la_io, a11, a12, kb, bc0, bc1, f0, la_io};
 #endif
   // (a11, a12, 1 - a11) = frc^2 A_tt / trace and kb = frc / trace come ready-made from the contact record (contact_rows);
   // kb = 0 marks a singular block
